@@ -5,6 +5,7 @@
     python bench.py --impl reference --steps K --warmup W    # the reference algorithm on the host CPU cores (oracle port)
     python bench.py --config cfg4                            # DPRNN-TasNet (segment / overlap-add path), its own line
     python bench.py --train [--n-sources 3 --batch 8]        # the training step alone, its own line
+    python bench.py ... --dump-outputs DIR                   # also write what the last timed step returned, as DIR/<name>.npy
 
 Workload (BASELINE.json configs[1], "cfg2"): Conv-TasNet N=512 L=16 B=128 H=512 Sc=128 P=3 X=8 R=3, gLN, 2 speakers,
 batch 32 x 4 s @ 8 kHz per GPU (weak scaling: every rank gets its own batch of 32; no data-path collective).
@@ -59,7 +60,12 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-train-block", action="store_true")
     ap.add_argument("--train", action="store_true", help="time the TRAINING step only; prints its own line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (rank 0; inputs are seeded, so two "
+                         "builds run with the same arguments can be compared output for output)")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes what the sm_100a path computed; it does not apply to --impl reference")
     d = {"cfg2": (32, 4.0, 8000, 2), "cfg3": (8, 4.0, 8000, 3), "cfg4": (16, 4.0, 8000, 2), "cfg5": (16, 8.0, 16000, 4)}[a.config]
     a.batch = a.batch if a.batch is not None else d[0]
     a.seconds = a.seconds if a.seconds is not None else d[1]
@@ -150,6 +156,27 @@ class ClockSampler:
                     reasons.add(name)
         sm.sort()
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": mx or None, "reasons": sorted(reasons), "samples": len(sm)}
+
+
+DUMP_BYTES = 60 * 2 ** 20   # data budget of --dump-outputs; the .npy headers fit in what is left of 64 MB
+
+
+def dump_outputs(path, arrays):
+    """Writes each tensor of `arrays` as <path>/<name>.npy: floating point as float32 (float64 stays float64), integers as float64
+    (exact).  Smallest first, every array gets an equal share of what is left of DUMP_BYTES; one larger than its share keeps every
+    k-th element of its flattened values, the same elements on every run."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    items = sorted(arrays.items(), key=lambda kv: kv[1].numel())
+    left = DUMP_BYTES
+    for i, (name, t) in enumerate(items):
+        a = t.detach().cpu().numpy()
+        a = a.astype(np.float64 if a.dtype == np.float64 or a.dtype.kind in "iub" else np.float32)
+        share = max(1, left // (len(items) - i) // a.itemsize)
+        if a.size > share:
+            a = a.reshape(-1)[::-(-a.size // share)]
+        np.save(os.path.join(path, name + ".npy"), a)
+        left -= a.nbytes
 
 
 def workload_config(args, world):
@@ -255,9 +282,10 @@ def build_convtasnet(args, dev, torch, S):
     return m
 
 
-def train_leg(args, torch, N, D, dev, rank, world, S, B, steps, warmup):
+def train_leg(args, torch, N, D, dev, rank, world, S, B, steps, warmup, outputs=None):
     """Data-parallel training step (egs/wsj0-mix/common/src/driver.py:146-157): fwd_train + PIT + native backward + ONE gradient
-    all-reduce + native global-norm clip + Adam.  Returns the `train` block."""
+    all-reduce + native global-norm clip + Adam.  Returns the `train` block; fills `outputs`, if given, with the loss of the last
+    timed step and the parameters it left (flattened, in named_parameters order)."""
     from ctn_b200.criterion.sdr import NegSISDR
     from ctn_b200.criterion.pit import PIT1d
     from ctn_b200.optim import FlatClipAdam
@@ -287,6 +315,9 @@ def train_leg(args, torch, N, D, dev, rank, world, S, B, steps, warmup):
     launches = model.last_launches + model.last_bwd_launches + opt.launches_per_step
     ar_ev.clear()
     ms, _, (loss, nel) = cuda_time(step, steps, torch, D, dev)
+    if outputs is not None:
+        outputs["loss"] = loss.detach()
+        outputs["params"] = torch.cat([p.detach().flatten() for p in model.parameters()])
     ar_ms = D.max_over_ranks(sum(a.elapsed_time(b) for a, b in ar_ev) / max(1, len(ar_ev)), dev)
     return {"workload": f"cfg3 per-GPU shape: Conv-TasNet {S}spk paper hparams, batch {B} x {args.seconds:g}s@{args.sample_rate // 1000}kHz per GPU, "
                         "fwd_train + PIT + backward + all-reduce + clip(5.0) + Adam(1e-3)", "global_batch": world * B,
@@ -366,8 +397,11 @@ def main():
     math_name = args.math or ("f16x3" if N.ctn_has_tcgen05() else "fp32")
 
     if args.train:
-        blk = train_leg(args, torch, N, D, dev, rank, world, S, B, args.steps, args.warmup)
+        outputs = {} if args.dump_outputs and rank == 0 else None
+        blk = train_leg(args, torch, N, D, dev, rank, world, S, B, args.steps, args.warmup, outputs)
         if rank == 0:
+            if outputs is not None:
+                dump_outputs(args.dump_outputs, outputs)
             print(json.dumps({"mode": "train", "metric": "audio-sec/s Conv-TasNet TRAIN step", "value": blk["audio_s_per_s"], "unit": "audio-sec/s",
                               "n_gpus": world, "steps": args.steps, "warmup": max(args.warmup, 2), "ms_per_step": blk["ms_per_step"],
                               "higher_is_better": True, "scaling": "weak", "dtype": math_name, "data": "synthetic", "config": {"workload": blk["workload"]},
@@ -396,7 +430,8 @@ def main():
 
     def step_resident():
         out = model(mixture_d)
-        return crit(out, sources_d)
+        loss, perm = crit(out, sources_d)
+        return out, loss, perm
 
     if args.config == "cfg4":
         loss_pin = torch.empty(1).pin_memory()
@@ -421,7 +456,7 @@ def main():
 
     with torch.no_grad():
         for _ in range(max(args.warmup, 3)):
-            loss, perm = step_resident()
+            step_resident()
         launches_per_step = getattr(model, "last_launches", 0) + N.ctn_last_launch_count()
         if args.config == "cfg4":   # the DPRNN path is made of many entry calls: count one whole step
             n0 = N.ctn_total_launch_count()
@@ -431,7 +466,10 @@ def main():
         # ---- timed: device-resident, stage timers OFF ---------------------------------------------------------
         N.ctn_profile_enable(0)
         with ClockSampler(local_rank) as clk:
-            ms, ms_local, _ = cuda_time(step_resident, args.steps, torch, D, dev)
+            ms, ms_local, last = cuda_time(step_resident, args.steps, torch, D, dev)
+        outputs = None
+        if args.dump_outputs and rank == 0:   # copied now: the calls below may reuse the device buffers
+            outputs = {name: t.cpu() for name, t in zip(("estimates", "loss", "perm"), last)}
         # ---- timed: end to end ----------------------------------------------------------------------------------
         for _ in range(2):
             step_e2e()
@@ -580,6 +618,8 @@ def main():
         # bounded sample: the full per-GPU batch, 1 warm-up + 2 timed steps (~ 20-30 s of CPU work at cfg2)
         leg = cpu_reference_leg(args, steps=2, warmup=1, cpu_batch=args.cpu_batch or args.batch)
         line["cpu_baseline"] = {k: leg[k] for k in ("value", "unit", "cores", "kind", "sample")}
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line), flush=True)
     if world > 1:
         import torch.distributed as dist
