@@ -215,18 +215,6 @@ static int run_tcn(const ctn_config_t* c, const ctn_block_params_t* blocks, TcnW
     CTN_TRY(rc);
   }
   const bool scaled = c->math == CTN_MATH_F16X3;
-  // Sample groups: the blocks are walked group by group (G samples through all R*X blocks, then the next G).  The hidden tensor h
-  // of a group (G * H * pitch * 4 bytes = 8.4 MB per sample at cfg2) is written by pw1 and read by pw2 a few hundred microseconds
-  // later from the SAME buffer for every group and block, so it stays resident in the 126 MB L2 instead of making a round trip
-  // through HBM (12.6 GB of the 24 GB a cfg2 step moved).  Every mixture is independent, so the arithmetic is unchanged.
-  static const char* env_grp = getenv("CTN_TCN_GROUP");
-  int G = env_grp ? atoi(env_grp) : 0;
-  if (G <= 0 || G > B || c->math == CTN_MATH_FP32) G = B;
-  for (int g0 = 0; g0 < B; g0 += G) {
-  const int Bg = B - g0 < G ? B - g0 : G;
-  const size_t go = (size_t)g0 * pitch;  // sample offset in rows of `pitch` floats, times the tensor's channel count
-  float* hbuf = ws->h;                   // one group-sized region, reused by every group
-  float* ubuf = ws->u;
   for (int r = 0; r < R; ++r) {
     for (int l = 0; l < X; ++l) {
       const int i = r * X + l;
@@ -234,22 +222,21 @@ static int run_tcn(const ctn_config_t* c, const ctn_block_params_t* blocks, TcnW
       const bool has_out = p.out_w != nullptr;
       if (!has_out && !(r == R - 1 && l == X - 1)) return CTN_EINVAL;
       const int dilation = dil ? dil[i] : (1 << l);  // dilated=True (tdcn.py:52-54)
-      double* st1 = ws->stats + (size_t)(2 * i) * B * 2 + 2 * g0;
-      double* st2 = ws->stats + (size_t)(2 * i + 1) * B * 2 + 2 * g0;
+      double* st1 = ws->stats + (size_t)(2 * i) * B * 2;
+      double* st2 = ws->stats + (size_t)(2 * i + 1) * B * 2;
       // K_A: h = PReLU(W1 x + b1), stats1
       PwArgs a;
       memset(&a, 0, sizeof(a));
       // tcgen05 modes: the residual stream ping-pongs between ws->x and ws->xalt; block i >= 1 applies block i-1's
       // update x += rstd2*r[:Bc] + c inside its own producer (PRO_RES) -- no separate finishing pass over x
       const bool fuse_res = c->math != CTN_MATH_FP32;
-      float* xbuf[2] = {ws->x + go * Bc, ws->xalt + go * Bc};
-      if (hooks) {  // per-block buffers: x_i is read from x_keep[i] (written by block i-1 below), kept for the backward
-        if (!fuse_res || g0 != 0) return CTN_EUNSUPPORTED;
-        hbuf = hooks->hpre[i];
-      }
+      float* xbuf[2] = {ws->x, ws->xalt};
+      // training forward: per-block buffers; x_i is read from x_keep[i] (written by block i-1 below), kept for the backward
+      if (hooks && !fuse_res) return CTN_EUNSUPPORTED;
+      float* const hbuf = hooks ? hooks->hpre[i] : ws->h;
       a.A = fuse_res ? xbuf[(i + 1) & 1] : xbuf[0];
       if (fuse_res && i == 0) a.A = hooks ? hooks->x_keep[0] : xbuf[0];
-      a.W = p.bottleneck_w; a.D = hbuf; a.B = Bg; a.M = H; a.K = Bc; a.frames = frames; a.pitch = pitch;
+      a.W = p.bottleneck_w; a.D = hbuf; a.B = B; a.M = H; a.K = Bc; a.frames = frames; a.pitch = pitch;
       a.store_pre = hooks ? 1 : 0;
       a.bias = p.bottleneck_b; a.slope = p.prelu1; a.stats_out = st1; a.wimg = ws->wimg1[i];
       if (scaled) a.act_scale = ws->scales + 2 * i;
@@ -258,15 +245,15 @@ static int run_tcn(const ctn_config_t* c, const ctn_block_params_t* blocks, TcnW
         // x_{i} = x_{i-1} + deferred gLN2 of block i-1;  x_{i-1} lives in xbuf[(i-1)&1], x_i goes to xbuf[i&1]
         pro1 = PRO_RES;
         a.A = hooks ? hooks->x_keep[i - 1] : xbuf[(i - 1) & 1];
-        a.res_r = ws->rblk[i - 1] + go * (Bc + Sc); a.res_Mt = Bc + Sc;  // block i-1 always has the out head (only the last block lacks it)
+        a.res_r = ws->rblk[i - 1]; a.res_Mt = Bc + Sc;  // block i-1 always has the out head (only the last block lacks it)
         a.res_v1 = ws->folds[i - 1].v1; a.res_v2 = ws->folds[i - 1].v2;
-        a.res_stats = ws->stats + (size_t)(2 * (i - 1) + 1) * B * 2 + 2 * g0; a.res_n = (double)H * (double)frames; a.res_eps = c->eps_tcn;
+        a.res_stats = ws->stats + (size_t)(2 * (i - 1) + 1) * B * 2; a.res_n = (double)H * (double)frames; a.res_eps = c->eps_tcn;
         a.res_x_out = hooks ? hooks->x_keep[i] : xbuf[i & 1];
       }
       if (hooks && !(c->math == CTN_MATH_F16X3 && ctn_pw_tma_supported(a, pro1, EPI_H))) return CTN_EUNSUPPORTED;
       { StageTimer tm(CTN_ST_PW1, st); CTN_TRY(pw_dispatch(a, pro1, EPI_H, c->math, st)); }
       const int Mt = has_out ? Bc + Sc : Sc;
-      float* rb = ws->rblk[i] + go * Mt;
+      float* rb = ws->rblk[i];
       const int pad_left = c->causal ? (c->sep_kernel - 1) * dilation : ((c->sep_kernel - 1) * dilation) / 2;
       // fused depthwise producer: 3 taps at dilation 1, 2 or a multiple of 4 (128-bit aligned tap loads); anything else runs the
       // stand-alone depthwise stage
@@ -276,7 +263,7 @@ static int run_tcn(const ctn_config_t* c, const ctn_block_params_t* blocks, TcnW
         // it straight to the tensor core; u never touches HBM.  r = [Wo;Ws] diag(gamma2) u
         StageTimer tm(CTN_ST_PW2, st);
         memset(&a, 0, sizeof(a));
-        a.A = hbuf; a.W = ws->folds[i].Wf; a.D = rb; a.B = Bg; a.M = Mt; a.K = H; a.frames = frames; a.pitch = pitch;
+        a.A = hbuf; a.W = ws->folds[i].Wf; a.D = rb; a.B = B; a.M = Mt; a.K = H; a.frames = frames; a.pitch = pitch;
         a.wimg = ws->wimg2[i];
         a.pro_slope = p.prelu2; a.dw_norm_g = p.norm1_g; a.dw_norm_b = p.norm1_b; a.dw_w = p.dw_w; a.dw_b = p.dw_b;
         a.dw_stats_in = st1; a.dw_stats_out = st2; a.dw_dilation = dilation; a.dw_pad_left = pad_left; a.dw_eps = c->eps_tcn;
@@ -290,11 +277,11 @@ static int run_tcn(const ctn_config_t* c, const ctn_block_params_t* blocks, TcnW
         if (hooks) return CTN_EUNSUPPORTED;
         // K_B: u = PReLU(dwconv(gLN1(h))), stats2
         { StageTimer tm(CTN_ST_DW, st);
-          CTN_TRY(ctn_dw_fwd(hbuf, ubuf, p.norm1_g, p.norm1_b, p.dw_w, p.dw_b, p.prelu2, st1, st2, Bg, H, frames, pitch,
+          CTN_TRY(ctn_dw_fwd(hbuf, ws->u, p.norm1_g, p.norm1_b, p.dw_w, p.dw_b, p.prelu2, st1, st2, B, H, frames, pitch,
                              c->sep_kernel, dilation, c->causal, c->eps_tcn, st)); }
         // K_C: r = [Wo;Ws] diag(gamma2) u
         memset(&a, 0, sizeof(a));
-        a.A = ubuf; a.W = ws->folds[i].Wf; a.D = rb; a.B = Bg; a.M = Mt; a.K = H; a.frames = frames; a.pitch = pitch;
+        a.A = ws->u; a.W = ws->folds[i].Wf; a.D = rb; a.B = B; a.M = Mt; a.K = H; a.frames = frames; a.pitch = pitch;
         a.wimg = ws->wimg2[i];
         if (scaled) a.act_scale = ws->scales + 2 * i + 1;
         { StageTimer tm(CTN_ST_PW2, st); CTN_TRY(pw_dispatch(a, PRO_NONE, EPI_RAW, c->math, st)); }
@@ -302,11 +289,10 @@ static int run_tcn(const ctn_config_t* c, const ctn_block_params_t* blocks, TcnW
       // K_F: residual update with the deferred gLN2 (x += rstd2*r[:Bc] + c); the skip rows are reduced once at the end
       if (has_out && c->math == CTN_MATH_FP32) {
         StageTimer tm(CTN_ST_FIN, st);
-        CTN_TRY(ctn_finish_fwd(rb, ws->folds[i], st2, (double)H * (double)frames, c->eps_tcn, xbuf[0], ws->skip + go * Sc, Bg, Bc,
+        CTN_TRY(ctn_finish_fwd(rb, ws->folds[i], st2, (double)H * (double)frames, c->eps_tcn, xbuf[0], ws->skip, B, Bc,
                                Sc, 1, 2 /* x rows only */, frames, pitch, st));
       }
     }
-  }
   }
   {
     StageTimer tm(CTN_ST_FIN, st);
@@ -804,29 +790,4 @@ extern "C" int ctn_convtasnet_loss_host(const ctn_config_t* cfg, const ctn_param
   if ((e = cudaMemcpyAsync(loss_mean_host, io.loss_mean, sizeof(float), cudaMemcpyDeviceToHost, st)) != cudaSuccess) return (int)e;
   if ((e = cudaMemcpyAsync(perm_host, io.perm, sizeof(int64_t) * (size_t)B * S, cudaMemcpyDeviceToHost, st)) != cudaSuccess) return (int)e;
   return CTN_OK;
-}
-
-// ------------------------------------------------------------------------------------------------
-// test hook
-// ------------------------------------------------------------------------------------------------
-extern "C" int ctn_debug_pointwise(const float* A, const float* W, float* D, int B, int M, int K, int frames, int pitch,
-                                   const float* bias, const float* slope, double* stats_out, int epi, int math,
-                                   const uint32_t* dbg, void* workspace, size_t workspace_bytes, ctn_stream_t stream) {
-  LaunchScope scope(A);
-  if (!A || !W || !D || B <= 0 || M <= 0 || K <= 0 || frames <= 0 || pitch < frames || pitch % 128 != 0) return CTN_EINVAL;
-  if (epi != EPI_RAW && epi != EPI_H) return CTN_EUNSUPPORTED;
-  if (epi == EPI_H && (!bias || !slope || !stats_out)) return CTN_EINVAL;
-  cudaStream_t st = (cudaStream_t)stream;
-  PwArgs a;
-  memset(&a, 0, sizeof(a));
-  a.A = A; a.W = W; a.D = D; a.B = B; a.M = M; a.K = K; a.frames = frames; a.pitch = pitch;
-  a.bias = bias; a.slope = slope; a.stats_out = stats_out;
-  if (math == CTN_MATH_FP32) return ctn_pw_simt(a, PRO_NONE, epi, st);
-  const size_t need = ctn_umma_wimg_bytes(M, K, math) + 512;
-  if (!workspace || workspace_bytes < need) return CTN_EWORKSPACE;
-  float* wimg = (float*)(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
-  CTN_TRY(ctn_umma_build_wimg(W, M, K, math, wimg, st));
-  a.wimg = wimg;
-  if (dbg) { a.dbg_idesc = dbg[0]; a.dbg_lbo_a = dbg[1]; a.dbg_sbo_a = dbg[2]; a.dbg_sbo_w = dbg[3]; }
-  return ctn_pw_umma(a, PRO_NONE, epi, math, st);
 }

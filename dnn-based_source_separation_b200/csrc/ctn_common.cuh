@@ -45,6 +45,16 @@ static inline int ctn_current_device() {
   cudaGetDevice(&d);
   return (d >= 0 && d < CTN_MAX_DEVICES) ? d : 0;
 }
+// SM count of the current device (persistent grids are sized by it), queried once per device ordinal
+inline int ctn_num_sms() {
+  static int sms[CTN_MAX_DEVICES] = {};
+  const int dev = ctn_current_device();
+  if (sms[dev] <= 0) {
+    cudaDeviceGetAttribute(&sms[dev], cudaDevAttrMultiProcessorCount, dev);
+    if (sms[dev] <= 0) sms[dev] = 148;
+  }
+  return sms[dev];
+}
 
 #define CTN_RETURN_IF_CUDA_ERR()                      \
   do {                                                \

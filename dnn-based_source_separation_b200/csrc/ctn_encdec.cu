@@ -149,9 +149,8 @@ static int launch_encoder(const float* x, const float* W, float* w, int B, int T
     if (e != cudaSuccess) return (int)e;
   }
   dim3 grid((pitch + 127) / 128, B);
-  static const char* env_v4 = getenv("CTN_ENC_V4");
   if constexpr (L <= 20) {  // longer kernels: the 3*stride + L input window no longer fits the register file
-  if (stride * 2 == L && pitch % 128 == 0 && (((uintptr_t)w) & 15) == 0 && !(env_v4 && atoi(env_v4) == 0)) {
+  if (stride * 2 == L && pitch % 128 == 0 && (((uintptr_t)w) & 15) == 0) {
     if (smem > 48 * 1024) {
       cudaError_t e = cudaFuncSetAttribute(k_encoder_v4<L, L / 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
       if (e != cudaSuccess) return (int)e;

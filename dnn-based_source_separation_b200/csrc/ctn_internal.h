@@ -72,8 +72,19 @@ struct PwArgs {
   // applies PReLU(dw_in_slope) on load; the depthwise pre-activation u_pre is stored to dw_u_pre_out (B, K, pitch)
   const float* dw_in_slope;
   float* dw_u_pre_out;
-  uint32_t dbg_idesc, dbg_lbo_a, dbg_sbo_a, dbg_sbo_w;  // 0 = defaults (descriptor probing from the debug entry)
 };
+
+// Output channels per n-tile (UMMA N) of the tcgen05 pointwise kernels.  The weight images are laid out in n-tiles of this width,
+// so the image builders and both kernel families use this one rule.
+__host__ __device__ inline int pick_n_tile(int M) { return M >= 256 ? 256 : ((M + 15) / 16) * 16; }
+// the fp16-piece mode keeps one scale per padded output channel in shared memory: contractions with more than
+// CTN_F16_MAX_ROWS padded output channels use the tf32 pieces instead (images and kernel are chosen by the same rule)
+constexpr int CTN_F16_MAX_ROWS = 2048;
+__host__ __device__ inline int eff_math(int M, int math) {
+  if (math != CTN_MATH_F16X3) return math;
+  const int n_tile = pick_n_tile(M);
+  return ((M + n_tile - 1) / n_tile) * n_tile > CTN_F16_MAX_ROWS ? CTN_MATH_TF32X3 : math;
+}
 
 // fp32 CUDA-core path (ctn_tcn_simt.cu)
 int ctn_pw_simt(const PwArgs& a, int pro, int epi, cudaStream_t st);

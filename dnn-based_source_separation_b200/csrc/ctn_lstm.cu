@@ -1200,10 +1200,7 @@ extern "C" int ctn_bilstm_proj_fwd(const float* z, int NSEQ, int T, int F, int H
   if (workspace_bytes < p.total) return CTN_EWORKSPACE;
   if (p.pair && !getenv("CTN_LSTM_PAIR")) {
     // the 2-CTA form halves the time of a step but needs twice the CTAs: worth it only while they all fit on the GPU at once
-    static int sms[CTN_MAX_DEVICES] = {};
-    const int dev = ctn_current_device();
-    if (!sms[dev]) cudaDeviceGetAttribute(&sms[dev], cudaDevAttrMultiProcessorCount, dev);
-    if (4 * ((NSEQ + LM - 1) / LM) > sms[dev] && !lstm_plan(F, H, w_fc ? Fo : 0, p, false)) return CTN_EUNSUPPORTED;
+    if (4 * ((NSEQ + LM - 1) / LM) > ctn_num_sms() && !lstm_plan(F, H, w_fc ? Fo : 0, p, false)) return CTN_EUNSUPPORTED;
   }
   if ((((uintptr_t)z) | ((uintptr_t)P) | ((uintptr_t)hout) | ((uintptr_t)workspace)) & 15) return CTN_EALIGN;
   cudaStream_t st = (cudaStream_t)stream;

@@ -23,7 +23,6 @@
 //   then   epilogue group 1 (EPI_H kernels: 4 more warps, upper half of the columns)
 #include <cuda.h>
 #include <cuda_fp16.h>
-#include <stdlib.h>
 #include <string.h>
 #include "ctn_internal.h"
 #include "ctn_umma_ptx.cuh"
@@ -52,10 +51,8 @@ struct TmaArgs {
   int op_stages, raw_stages;
   uint32_t op_stage_bytes, raw_stage_bytes, raw_tx_bytes, w_bytes, hdr_bytes, res_tab_off, idesc;
   int reverse;   // walk the (sample, time tile) list backwards
-  int pair;      // 1: clusters of 2 CTAs, cta_group::2 MMAs (each CTA stages half of every weight slab)
   int dw_three;  // PRO_DW: 0 = one window box of 128 + 2*dw_pad frames, 1 = three boxes of 128 frames at t-d, t, t+d
   int dw_pad;    // window mode: halo frames on each side (dilation rounded up to a multiple of 4)
-  uint32_t dbg;
 };
 
 template <int PRO> struct Roles {
@@ -102,10 +99,7 @@ __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* tm) {
 
 // DWM (PRO_DW only): depthwise tap geometry fixed at compile time -- 1 / 2: dilation 1 / 2 in the aligned window [t-4, t+8);
 // 3: dilation >= 4, one window box of 128 + 2d frames; 4: dilation >= 128, three boxes of 128 frames.  0 for the other prologues.
-// PAIR: the kernel runs as clusters of 2 CTAs driving tcgen05 cta_group::2 MMAs (M = 256 = two time tiles): each CTA stages its own
-// activation tile and HALF of every weight slab, so the weight bytes written to and read from shared memory per CTA halve (the
-// shared-memory port was ~90 % busy in the single-CTA kernel: LDS/STS 41 %, TMA + bulk writes 23 %, tensor-core operand reads 27 %).
-template <int PRO, int EPI, int DWM, bool PAIR>
+template <int PRO, int EPI, int DWM>
 __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_tma(const __grid_constant__ TmaArgs g) {
   constexpr bool TRAIN = (DWM & 8) != 0;  // training forward: PReLU on load, u_pre stored (see PwArgs::dw_in_slope)
   constexpr int DCLS = (DWM & 7) == 1 ? 1 : ((DWM & 7) == 2 ? 2 : 4);
@@ -126,8 +120,7 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_tma(const __grid_
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < g.op_stages; ++s) {
-      // pair mode: the peer's relay warp forwards "my stage s is full" to the leader's full[s] with one more arrival
-      ptx::mbar_init(ptx::smem_u32(&hdr->full[s]), PROD_WARPS + 1 + ((PAIR && ptx::cluster_ctarank() == 0) ? 1 : 0));
+      ptx::mbar_init(ptx::smem_u32(&hdr->full[s]), PROD_WARPS + 1);
       ptx::mbar_init(ptx::smem_u32(&hdr->empty[s]), 1);
     }
     for (int s = 0; s < g.raw_stages; ++s) {
@@ -136,14 +129,11 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_tma(const __grid_
     }
     for (int i = 0; i < 2; ++i) {
       ptx::mbar_init(ptx::smem_u32(&hdr->tfull[i]), 1);
-      ptx::mbar_init(ptx::smem_u32(&hdr->tempty[i]), PAIR ? 2 * 4 * EGROUPS : 128 * EGROUPS);  // pair: one arrival per epilogue warp of both CTAs
+      ptx::mbar_init(ptx::smem_u32(&hdr->tempty[i]), 128 * EGROUPS);
     }
     ptx::fence_mbar_init();
   }
-  if (warp == 4) {
-    if constexpr (PAIR) ptx::tmem_alloc2(ptx::smem_u32(&hdr->tmem_base), 512);
-    else ptx::tmem_alloc(ptx::smem_u32(&hdr->tmem_base), 512);
-  }
+  if (warp == 4) ptx::tmem_alloc(ptx::smem_u32(&hdr->tmem_base), 512);
   if (warp == 5 && lane == 0) {
     tma_prefetch_desc(&g.tmA);
     if (PRO == PRO_RES) tma_prefetch_desc(&g.tmR);
@@ -165,36 +155,27 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_tma(const __grid_
   __syncthreads();
   ptx::tc_fence_after();
   const uint32_t tmem_base = hdr->tmem_base;
-  if (PAIR) ptx::cluster_sync_all();  // barriers of both CTAs initialised before any remote arrive / multicast commit
-  const int crank = PAIR ? (int)ptx::cluster_ctarank() : 0;
-  constexpr int CL = PAIR ? 2 : 1;
-  const int cidx = (int)blockIdx.x / CL, ncl = (int)gridDim.x / CL;
 
   // EPI_MASKDEC: a CTA walks ALL n-tiles of a (sample, time tile) back to back (the decoder sums over the channels of a source
   // in registers); the other kernels interleave n-tiles across CTAs (n-tile fastest, co-running CTAs share activations in L2)
-  // Work: a cluster (1 or 2 CTAs) walks cluster items; rank r of the cluster takes time tile L = group * CL + r.  Ranks whose L
-  // falls off the end run a dummy tile (TMA zero-fills the out-of-range rows; nothing is stored or counted).
   const int tiles_total = g.num_items / g.n_tiles;
-  const int groups_total = (tiles_total + CL - 1) / CL;
-  const int items_per_cta = EPI == EPI_MASKDEC ? ((groups_total - cidx + ncl - 1) / ncl) * g.n_tiles
-                                               : (groups_total * g.n_tiles - cidx + ncl - 1) / ncl;
-  auto decode = [&](int it2, int& nt2, int& tt2, int& b2) -> bool {
-    int Lg;
+  const int cta = (int)blockIdx.x, ncta = (int)gridDim.x;
+  const int items_per_cta = EPI == EPI_MASKDEC ? ((tiles_total - cta + ncta - 1) / ncta) * g.n_tiles
+                                               : (g.num_items - cta + ncta - 1) / ncta;
+  auto decode = [&](int it2, int& nt2, int& tt2, int& b2) {
+    int L;
     if (EPI == EPI_MASKDEC) {
       nt2 = it2 % g.n_tiles;
-      Lg = cidx + (it2 / g.n_tiles) * ncl;
+      L = cta + (it2 / g.n_tiles) * ncta;
     } else {
-      const int J = cidx + it2 * ncl;
+      const int J = cta + it2 * ncta;
       nt2 = J % g.n_tiles;
-      Lg = J / g.n_tiles;
+      L = J / g.n_tiles;
     }
-    int L = Lg * CL + crank;
-    const bool in_range = L < tiles_total;
     // reverse walk (pw2): the previous kernel (pw1, forward) wrote the LAST samples' h most recently -- start with what is still in L2
-    if (g.reverse && in_range) L = tiles_total - 1 - L;
+    if (g.reverse) L = tiles_total - 1 - L;
     tt2 = L % g.t_tiles;
     b2 = L / g.t_tiles;
-    return in_range;
   };
   if (EPI == EPI_MASKDEC) {
     // decoder basis (Nb x 16 taps) resident in shared memory behind the raw ring, then the [2][128][16] combine buffer
@@ -220,41 +201,26 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_tma(const __grid_
             const uint32_t dst = raw0 + (uint32_t)rs * g.raw_stage_bytes;
             const int c = ks * KS + sub * RC;  // first channel of the stage
             ptx::mbar_arrive_expect_tx(fb, g.raw_tx_bytes);
-            if (!(g.dbg & 2u)) {
-              if (PRO == PRO_DW) {
-                if (THREE) {
+            if (PRO == PRO_DW) {
+              if (THREE) {
 #pragma unroll
-                  for (int k = 0; k < 3; ++k)
-                    tma_load_2d(dst + (uint32_t)k * (RC * TM * 4), &g.tmA, tt * TM + (k - 1) * a.dw_dilation, b * a.K + c, fb);
-                  ptx::bulk_g2s(dst + 3u * (RC * TM * 4), g.dwp + (size_t)c * 8, RC * 32, fb);
-                } else {
-                  tma_load_2d(dst, &g.tmA, tt * TM - g.dw_pad, b * a.K + c, fb);
-                  ptx::bulk_g2s(dst + (uint32_t)(RC * (TM + 2 * g.dw_pad) * 4), g.dwp + (size_t)c * 8, RC * 32, fb);
-                }
+                for (int k = 0; k < 3; ++k)
+                  tma_load_2d(dst + (uint32_t)k * (RC * TM * 4), &g.tmA, tt * TM + (k - 1) * a.dw_dilation, b * a.K + c, fb);
+                ptx::bulk_g2s(dst + 3u * (RC * TM * 4), g.dwp + (size_t)c * 8, RC * 32, fb);
               } else {
-                tma_load_2d(dst, &g.tmA, tt * TM, b * a.K + c, fb);
-                if (PRO == PRO_RES) tma_load_2d(dst + RC * TM * 4, &g.tmR, tt * TM, b * a.res_Mt + c, fb);
+                tma_load_2d(dst, &g.tmA, tt * TM - g.dw_pad, b * a.K + c, fb);
+                ptx::bulk_g2s(dst + (uint32_t)(RC * (TM + 2 * g.dw_pad) * 4), g.dwp + (size_t)c * 8, RC * 32, fb);
               }
             } else {
-              // debug: no activation loads -- complete the transaction count by hand
-              asm volatile("mbarrier.complete_tx.relaxed.cta.shared::cta.b64 [%0], %1;" ::"r"(fb), "r"(g.raw_tx_bytes) : "memory");
+              tma_load_2d(dst, &g.tmA, tt * TM, b * a.K + c, fb);
+              if (PRO == PRO_RES) tma_load_2d(dst + RC * TM * 4, &g.tmR, tt * TM, b * a.res_Mt + c, fb);
             }
             if (++rs == g.raw_stages) { rs = 0; rph ^= 1u; }
           }
           ptx::mbar_wait(ptx::smem_u32(&hdr->empty[s]), ph ^ 1u);
           const uint32_t fb = ptx::smem_u32(&hdr->full[s]);
-          if constexpr (!PAIR) {
-            ptx::mbar_arrive_expect_tx(fb, 2 * g.w_bytes);
-            ptx::bulk_g2s(op0 + (uint32_t)s * g.op_stage_bytes + 2 * A_BYTES, wsrc + (size_t)ks * 2 * g.w_bytes, 2 * g.w_bytes, fb);
-          } else {
-            // this CTA stages rows [crank * n_tile/2, + n_tile/2) of the slab: a contiguous half of the hi image and of the lo image
-            const uint32_t half = g.w_bytes / 2;
-            ptx::mbar_arrive_expect_tx(fb, 2 * half);
-            const uint8_t* src = wsrc + (size_t)ks * 2 * g.w_bytes + (size_t)crank * half;
-            const uint32_t wdst = op0 + (uint32_t)s * g.op_stage_bytes + 2 * A_BYTES;
-            ptx::bulk_g2s(wdst, src, half, fb);
-            ptx::bulk_g2s(wdst + half, src + g.w_bytes, half, fb);
-          }
+          ptx::mbar_arrive_expect_tx(fb, 2 * g.w_bytes);
+          ptx::bulk_g2s(op0 + (uint32_t)s * g.op_stage_bytes + 2 * A_BYTES, wsrc + (size_t)ks * 2 * g.w_bytes, 2 * g.w_bytes, fb);
           if (++s == g.op_stages) { s = 0; ph ^= 1u; }
         }
       }
@@ -275,12 +241,11 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_tma(const __grid_
     const int dw_wd = TM + 2 * g.dw_pad;  // PRO_DW window mode: floats per channel row of a raw stage
     for (int it = 0; it < items_per_cta; ++it) {
       int nt, tt, b;
-      const bool live = decode(it, nt, tt, b);
-      const int bs = live ? b : 0;  // dummy tile of a pair: any valid sample for the statistics reads, nothing is stored
+      decode(it, nt, tt, b);
       float2 mr1 = make_float2(0.f, 1.f), mr_res = make_float2(0.f, 1.f);
       float2 dls = make_float2(0.f, 0.f), dlss = make_float2(0.f, 0.f);
-      if (PRO == PRO_DW) mr1 = gln_mean_rstd(a.dw_stats_in + 2 * bs, (double)a.K * (double)a.frames, a.dw_eps);
-      if (PRO == PRO_RES) mr_res = gln_mean_rstd(a.res_stats + 2 * bs, a.res_n, a.res_eps);
+      if (PRO == PRO_DW) mr1 = gln_mean_rstd(a.dw_stats_in + 2 * b, (double)a.K * (double)a.frames, a.dw_eps);
+      if (PRO == PRO_RES) mr_res = gln_mean_rstd(a.res_stats + 2 * b, a.res_n, a.res_eps);
       const int tbase = tt * TM + lane * 4;
       bool dw_interior = false;
       if (PRO == PRO_DW) {
@@ -331,7 +296,7 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_tma(const __grid_
               float4 upre;
               if (dw_interior && c < a.K) v[sub][j] = dw_channel<DCLS, true, TRAIN>(q0, q1, q2, gsc, gsh, w0, w1, w2, bd, pslope, first, tstep, tbase, a.frames, true, dls, dlss, &upre);
               else v[sub][j] = dw_channel<DCLS, false, TRAIN>(q0, q1, q2, gsc, gsh, w0, w1, w2, bd, pslope, first, tstep, tbase, a.frames, c < a.K, dls, dlss, &upre);
-              if (TRAIN && nt == 0 && live && c < a.K) {  // the taps carry the operand scale: undo it (power of two, exact)
+              if (TRAIN && nt == 0 && c < a.K) {  // the taps carry the operand scale: undo it (power of two, exact)
                 const float ia = 1.f / act_s;
                 *reinterpret_cast<float4*>(a.dw_u_pre_out + ((size_t)b * a.K + c) * a.pitch + tbase) =
                     make_float4(upre.x * ia, upre.y * ia, upre.z * ia, upre.w * ia);
@@ -355,7 +320,7 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_tma(const __grid_
                 if (tbase + 1 >= a.frames) x.y = 0.f;
                 if (tbase + 2 >= a.frames) x.z = 0.f;
                 if (tbase + 3 >= a.frames) x.w = 0.f;
-                if (nt == 0 && k < a.K && live) *reinterpret_cast<float4*>(a.res_x_out + ((size_t)b * a.K + k) * a.pitch + tbase) = x;
+                if (nt == 0 && k < a.K) *reinterpret_cast<float4*>(a.res_x_out + ((size_t)b * a.K + k) * a.pitch + tbase) = x;
                 dep += rr.x + rr.w;
               }
               dep += x.x + x.w;
@@ -398,7 +363,7 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_tma(const __grid_
         if (lane == 0) ptx::mbar_arrive(ptx::smem_u32(&hdr->full[s]));
         if (++s == g.op_stages) { s = 0; ph ^= 1u; }
       }
-      if (PRO == PRO_DW && nt == 0 && live) {
+      if (PRO == PRO_DW && nt == 0) {
         // the sums were taken over act_s * u: undo the power-of-two scale exactly in double
         const double inv = 1.0 / (double)act_s;
         const double sd = warp_sum_d((double)dls.x + (double)dls.y) * inv, ssd = warp_sum_d((double)dlss.x + (double)dlss.y) * inv * inv;
@@ -407,69 +372,42 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_tma(const __grid_
     }
   } else if (warp == 4) {
     // ===================================== MMA ISSUER =======================================================
-    if (!PAIR || crank == 0) {  // pair mode: only the leader CTA issues (its MMAs span both CTAs' shared memory and TMEM)
-      int s = 0;
-      uint32_t ph = 0;
-      const bool leader = ptx::elect_one();
-      const uint64_t da_t = ptx::make_smem_desc(0, 1024u, 2048u, 2u);  // A: MN-major SWIZZLE_128B (64-step atoms, 8-channel groups)
-      const uint64_t dw_t = ptx::make_smem_desc(0, 16u, 512u, 4u);     // W: K-major SWIZZLE_64B rows of 32 k
-      const uint32_t w_lo_off = (PAIR ? g.w_bytes / 2 : g.w_bytes) >> 4;  // pair: [hi half][lo half] of this CTA's rows
-      auto mma = [&](uint32_t d, uint64_t da, uint64_t dw, uint32_t accum) {
-        if constexpr (PAIR) ptx::mma2_f16(d, da, dw, g.idesc, accum);
-        else ptx::mma_f16(d, da, dw, g.idesc, accum);
-      };
-      auto commit = [&](uint64_t* bar) {
-        if constexpr (PAIR) ptx::mma2_commit_multicast(ptx::smem_u32(bar), (uint16_t)3u);  // same barrier in both CTAs
-        else ptx::mma_commit(ptx::smem_u32(bar));
-      };
-      for (int it = 0; it < items_per_cta; ++it) {
-        const int acc = it & 1;
-        if (PAIR) ptx::mbar_wait_cluster(ptx::smem_u32(&hdr->tempty[acc]), ((uint32_t)(it >> 1) & 1u) ^ 1u);
-        else ptx::mbar_wait(ptx::smem_u32(&hdr->tempty[acc]), ((uint32_t)(it >> 1) & 1u) ^ 1u);
+    int s = 0;
+    uint32_t ph = 0;
+    const bool leader = ptx::elect_one();
+    const uint64_t da_t = ptx::make_smem_desc(0, 1024u, 2048u, 2u);  // A: MN-major SWIZZLE_128B (64-step atoms, 8-channel groups)
+    const uint64_t dw_t = ptx::make_smem_desc(0, 16u, 512u, 4u);     // W: K-major SWIZZLE_64B rows of 32 k
+    for (int it = 0; it < items_per_cta; ++it) {
+      const int acc = it & 1;
+      ptx::mbar_wait(ptx::smem_u32(&hdr->tempty[acc]), ((uint32_t)(it >> 1) & 1u) ^ 1u);
+      ptx::tc_fence_after();
+      const uint32_t d_tmem = tmem_base + (uint32_t)acc * 256u;
+      int prev_s = -1;
+      for (int ks = 0; ks < g.k_slabs; ++ks) {
+        ptx::mbar_wait(ptx::smem_u32(&hdr->full[s]), ph);
         ptx::tc_fence_after();
-        const uint32_t d_tmem = tmem_base + (uint32_t)acc * 256u;
-        int prev_s = -1;
-        for (int ks = 0; ks < g.k_slabs; ++ks) {
-          if (PAIR) ptx::mbar_wait_cluster(ptx::smem_u32(&hdr->full[s]), ph);
-          else ptx::mbar_wait(ptx::smem_u32(&hdr->full[s]), ph);
-          ptx::tc_fence_after();
-          const uint32_t st_base = op0 + (uint32_t)s * g.op_stage_bytes;
-          const uint32_t a_hi = st_base >> 4, a_lo = (st_base + A_BYTES) >> 4;
-          const uint32_t w_hi = (st_base + 2 * A_BYTES) >> 4, w_lo = w_hi + w_lo_off;
-          if (leader) {
+        const uint32_t st_base = op0 + (uint32_t)s * g.op_stage_bytes;
+        const uint32_t a_hi = st_base >> 4, a_lo = (st_base + A_BYTES) >> 4;
+        const uint32_t w_hi = (st_base + 2 * A_BYTES) >> 4, w_lo = w_hi + (g.w_bytes >> 4);
+        if (leader) {
 #pragma unroll
-            for (int kk = 0; kk < KS / 16; ++kk) {
-              if (g.dbg & 8u) break;
-              const uint64_t da_hi = da_t | (uint64_t)(a_hi + kk * 256), dw_hi = dw_t | (uint64_t)(w_hi + kk * 2);
-              const uint64_t da_lo = da_t | (uint64_t)(a_lo + kk * 256), dw_lo = dw_t | (uint64_t)(w_lo + kk * 2);
-              mma(d_tmem, da_hi, dw_hi, (ks | kk) ? 1u : 0u);
-              if (kk == 0 && prev_s >= 0) commit(&hdr->empty[prev_s]);  // previous slab's stage
-              mma(d_tmem, da_lo, dw_hi, 1u);
-              mma(d_tmem, da_hi, dw_lo, 1u);
-            }
-            if ((g.dbg & 8u) && prev_s >= 0) commit(&hdr->empty[prev_s]);
-            if (ks == g.k_slabs - 1) {
-              commit(&hdr->empty[s]);
-              commit(&hdr->tfull[acc]);
-            }
+          for (int kk = 0; kk < KS / 16; ++kk) {
+            const uint64_t da_hi = da_t | (uint64_t)(a_hi + kk * 256), dw_hi = dw_t | (uint64_t)(w_hi + kk * 2);
+            const uint64_t da_lo = da_t | (uint64_t)(a_lo + kk * 256), dw_lo = dw_t | (uint64_t)(w_lo + kk * 2);
+            ptx::mma_f16(d_tmem, da_hi, dw_hi, g.idesc, (ks | kk) ? 1u : 0u);
+            if (kk == 0 && prev_s >= 0) ptx::mma_commit(ptx::smem_u32(&hdr->empty[prev_s]));  // previous slab's stage
+            ptx::mma_f16(d_tmem, da_lo, dw_hi, g.idesc, 1u);
+            ptx::mma_f16(d_tmem, da_hi, dw_lo, g.idesc, 1u);
           }
-          __syncwarp();
-          prev_s = s;
-          if (++s == g.op_stages) { s = 0; ph ^= 1u; }
+          if (ks == g.k_slabs - 1) {
+            ptx::mma_commit(ptx::smem_u32(&hdr->empty[s]));
+            ptx::mma_commit(ptx::smem_u32(&hdr->tfull[acc]));
+          }
         }
+        __syncwarp();
+        prev_s = s;
+        if (++s == g.op_stages) { s = 0; ph ^= 1u; }
       }
-    } else {
-      // peer CTA of a pair: forwards "my stage s is full" (its producer warps + its half of the weight slab) to the leader's
-      // full[s] with ONE cluster-scope arrival per slab
-      int s = 0;
-      uint32_t ph = 0;
-      for (int it = 0; it < items_per_cta; ++it)
-        for (int ks = 0; ks < g.k_slabs; ++ks) {
-          ptx::mbar_wait(ptx::smem_u32(&hdr->full[s]), ph);
-          if (lane == 0) ptx::mbar_arrive_remote(ptx::smem_u32(&hdr->full[s]), 0);
-          __syncwarp();
-          if (++s == g.op_stages) { s = 0; ph ^= 1u; }
-        }
     }
     __syncwarp();
   } else {
@@ -487,13 +425,12 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_tma(const __grid_
     for (int i = 0; i < 8; ++i) dacc[i] = make_float2(0.f, 0.f);
     for (int it = 0; it < items_per_cta; ++it) {
       int nt, tt, b;
-      const bool live = decode(it, nt, tt, b);
-      if (!live) { b = 0; tt = 0; }
+      decode(it, nt, tt, b);
       const int acc = it & 1;
       const int t = tt * TM + te;
-      const bool tvalid = t < a.frames && live;
+      const bool tvalid = t < a.frames;
       const int n0 = nt * g.n_tile;
-      const int nvalid = live ? min(g.n_tile, a.M - n0) : 0;  // dummy tile of a pair: nothing to read, store or count
+      const int nvalid = min(g.n_tile, a.M - n0);
       if (EPI == EPI_H || EPI == EPI_MASKDEC) {
         asm volatile("bar.sync 1, %0;" ::"n"(128 * EGROUPS) : "memory");  // previous item's readers are done with sp
         for (int i = tid_e; i < g.n_tile; i += 128 * EGROUPS) sp[i] = i < nvalid ? __ldg(a.bias + n0 + i) : 0.f;
@@ -508,8 +445,8 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_tma(const __grid_
       const int csplit = EGROUPS == 2 ? ((ncols_all / 2 + 15) & ~15) : ncols_all;
       const int cbeg = egroup == 0 ? 0 : csplit;
       const int ncols = egroup == 0 ? csplit : ncols_all;
-      const bool do_store = !(g.dbg & 1u);
-      const bool tile_full = tt * TM + TM <= a.frames;
+      // every time step of the tile is a real frame; `tvalid &&` is implied, and stating it keeps the PRO_DW kernels at 122 registers
+      const bool tile_full = tvalid && tt * TM + TM <= a.frames;
       // EPI_MASKDEC: w_hat[n][t] = w[n][t] * sigmoid(logit) is contracted on the spot with the decoder basis:
       //   full[8 t + k] += w_hat[n][t] * Dec[n][k], k < 16 (ConvTranspose1d(N,1,16,stride 8), filterbank.py:245-247), 16 partial
       // sums per thread (= per frame) in registers across the n-tiles of one source
@@ -547,7 +484,7 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_tma(const __grid_
       auto process = [&](const uint32_t (&buf)[16], const float (&wv)[16], int c0) {
         if (EPI == EPI_MASKDEC) { process_dec(buf, wv, c0); return; }
         float* q = Dp + (size_t)c0 * a.pitch;
-        const bool full = (c0 + 16 <= nvalid) && tile_full && do_store;  // warp-uniform
+        const bool full = (c0 + 16 <= nvalid) && tile_full;  // warp-uniform
         const float osc = ssc_all[n0 + c0];  // one power-of-two scale per 16-row weight group (and the operand scale)
         float o[16];
 #pragma unroll
@@ -582,7 +519,7 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_tma(const __grid_
           for (int j = 0; j < 16; ++j) {
             const float v = tvalid ? o[j] : 0.f;
             if (c0 + j < nvalid) {
-              if (do_store) q[(size_t)j * a.pitch] = v;
+              q[(size_t)j * a.pitch] = v;
               if (EPI == EPI_H) { const float sv = store_pre ? prelu_f(v, eslope) : v; ls += sv; lss = fmaf(sv, sv, lss); }
             }
           }
@@ -590,34 +527,25 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_tma(const __grid_
       };
       uint32_t bufA[16], bufB[16];
       float wvA[16], wvB[16];
-      const bool pf = EPI == EPI_MASKDEC && !(g.dbg & 32u);  // dbg 32: load at the point of use (A/B of the prefetch)
       if (EPI == EPI_MASKDEC && cbeg < ncols) load_w(wvA, cbeg);
       if (cbeg < ncols) ptx::tmem_ld16(taddr + (uint32_t)cbeg, bufA);
       for (int c0 = cbeg; c0 < ncols; c0 += 32) {
         ptx::tmem_ld_wait();
         if (c0 + 16 < ncols) {
           ptx::tmem_ld16(taddr + (uint32_t)(c0 + 16), bufB);
-          if (pf) load_w(wvB, c0 + 16);
+          if (EPI == EPI_MASKDEC) load_w(wvB, c0 + 16);
         }
         process(bufA, wvA, c0);
         ptx::tmem_ld_wait();
-        if (c0 + 32 < ncols) ptx::tmem_ld16(taddr + (uint32_t)(c0 + 32), bufA);
-        if (EPI == EPI_MASKDEC && !pf && c0 + 16 < ncols) load_w(wvB, c0 + 16);
-        if (pf && c0 + 32 < ncols) load_w(wvA, c0 + 32);
+        if (c0 + 32 < ncols) {
+          ptx::tmem_ld16(taddr + (uint32_t)(c0 + 32), bufA);
+          if (EPI == EPI_MASKDEC) load_w(wvA, c0 + 32);
+        }
         if (c0 + 16 < ncols) process(bufB, wvB, c0 + 16);
-        if (EPI == EPI_MASKDEC && !pf && c0 + 32 < ncols) load_w(wvA, c0 + 32);
       }
       ptx::tc_fence_before();
-      if (PAIR) {  // one arrival per warp, on the LEADER's barrier (its MMA warp overwrites both CTAs' accumulators)
-        __syncwarp();
-        if (lane == 0) {
-          if (crank == 0) ptx::mbar_arrive(ptx::smem_u32(&hdr->tempty[acc]));
-          else ptx::mbar_arrive_remote(ptx::smem_u32(&hdr->tempty[acc]), 0);
-        }
-      } else {
-        ptx::mbar_arrive(ptx::smem_u32(&hdr->tempty[acc]));
-      }
-      if (EPI == EPI_MASKDEC && (n0 + g.n_tile) % a.Nb == 0 && live) {
+      ptx::mbar_arrive(ptx::smem_u32(&hdr->tempty[acc]));
+      if (EPI == EPI_MASKDEC && (n0 + g.n_tile) % a.Nb == 0) {
         // last n-tile of source s: combine the two column halves (epilogue groups) and the two overlapping frames, crop
         // (conv_tasnet.py:169) and store.  Thread (group gq, frame te) owns samples 8 te + 4 gq .. +3 of the tile.
         float4* ab = reinterpret_cast<float4*>(accbuf + ((size_t)egroup * 128 + te) * 16);
@@ -659,7 +587,7 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_tma(const __grid_
         }
         asm volatile("bar.sync 1, %0;" ::"n"(128 * EGROUPS) : "memory");  // accbuf is reused by the next source
       }
-      if (EPI == EPI_H && live) {
+      if (EPI == EPI_H) {
         const double sd = warp_sum_d((double)ls), ssd = warp_sum_d((double)lss);
         if (lane == 0) { atomicAdd(&a.stats_out[2 * b], sd); atomicAdd(&a.stats_out[2 * b + 1], ssd); }
       }
@@ -668,11 +596,7 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_tma(const __grid_
   ptx::tc_fence_before();
   __syncthreads();
   ptx::tc_fence_after();
-  if (PAIR) ptx::cluster_sync_all();  // nobody exits while the peer may still arrive on / multicast into it
-  if (warp == 4) {
-    if constexpr (PAIR) ptx::tmem_dealloc2(tmem_base, 512);
-    else ptx::tmem_dealloc(tmem_base, 512);
-  }
+  if (warp == 4) ptx::tmem_dealloc(tmem_base, 512);
 }
 
 // ---- host side ----------------------------------------------------------------------------------------------------
@@ -703,73 +627,30 @@ int make_map(CUtensorMap* tm, const float* ptr, int rows, int pitch, int box_col
   return r == CUDA_SUCCESS ? CTN_OK : CTN_EINVAL;
 }
 
-int g_sms[CTN_MAX_DEVICES] = {0};
-int num_sms() {
-  const int dev = ctn_current_device();
-  if (g_sms[dev] == 0) {
-    cudaDeviceGetAttribute(&g_sms[dev], cudaDevAttrMultiProcessorCount, dev);
-    if (g_sms[dev] <= 0) g_sms[dev] = 148;
-  }
-  return g_sms[dev];
-}
-
-template <int PRO, int EPI, int DWM, bool PAIR>
-int launch1(const TmaArgs& g, size_t smem, int grid, cudaStream_t st) {
+template <int PRO, int EPI, int DWM = 0>
+int launch(const TmaArgs& g, size_t smem, int grid, cudaStream_t st) {
   static bool attr_done[CTN_MAX_DEVICES] = {false};
   const int dev = ctn_current_device();
   if (!attr_done[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(k_pw_tma<PRO, EPI, DWM, PAIR>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    cudaError_t e = cudaFuncSetAttribute(k_pw_tma<PRO, EPI, DWM>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     if (e != cudaSuccess) return (int)e;
     attr_done[dev] = true;
   }
-  if (PAIR) {  // a kernel that contains cta_group::2 instructions must be launched with an even cluster size
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3(grid & ~1);
-    cfg.blockDim = dim3(Roles<PRO>::THREADS);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, k_pw_tma<PRO, EPI, DWM, PAIR>, g);
-    if (e != cudaSuccess) return (int)e;
-    CTN_COUNT_LAUNCH();
-    CTN_RETURN_IF_CUDA_ERR();
-    return CTN_OK;
-  }
-  k_pw_tma<PRO, EPI, DWM, PAIR><<<grid, Roles<PRO>::THREADS, smem, st>>>(g);
+  k_pw_tma<PRO, EPI, DWM><<<grid, Roles<PRO>::THREADS, smem, st>>>(g);
   CTN_COUNT_LAUNCH();
   CTN_RETURN_IF_CUDA_ERR();
   return CTN_OK;
-}
-
-template <int PRO, int EPI, int DWM = 0>
-int launch(const TmaArgs& g, size_t smem, int grid, cudaStream_t st) {
-  return g.pair ? launch1<PRO, EPI, DWM, true>(g, smem, grid, st) : launch1<PRO, EPI, DWM, false>(g, smem, grid, st);
 }
 
 }  // namespace
 
 // 1 when (pro, epi, shape) is served by the TMA-fed kernels (fp16-piece mode only); the caller falls back to k_pw_umma otherwise
 int ctn_pw_tma_supported(const PwArgs& a, int pro, int epi) {
-  static const char* env = getenv("CTN_PW_TMA");
-  if (env && atoi(env) == 0) return 0;
-  if (!encode_fn() || getenv("CTN_UMMA_NTILE")) return 0;
-  {  // same rule as eff_math (ctn_umma.cu): more than 2048 padded output channels use the tf32 images
-    const int n_tile = a.M >= 256 ? 256 : ((a.M + 15) / 16) * 16;
-    if (((a.M + n_tile - 1) / n_tile) * n_tile > 2048) return 0;
-  }
+  if (!encode_fn() || eff_math(a.M, CTN_MATH_F16X3) != CTN_MATH_F16X3) return 0;  // fp16 weight images only
   if (!((pro == PRO_DW && epi == EPI_RAW) || ((pro == PRO_RES || pro == PRO_NONE) && epi == EPI_H) || (pro == PRO_PRELU && epi == EPI_MASKDEC)))
     return 0;
   if (epi == EPI_MASKDEC) {
-    static const char* envd = getenv("CTN_MASKDEC");
-    if (envd && atoi(envd) == 0) return 0;
-    const int n_tile = a.M >= 256 ? 256 : ((a.M + 15) / 16) * 16;
+    const int n_tile = pick_n_tile(a.M);
     if (!a.dec_w || a.Nb <= 0 || a.M % a.Nb != 0 || a.Nb % n_tile != 0 || a.Nb > 1024) return 0;  // whole n-tiles per source; basis fits smem
   }
   if (a.pitch % TM != 0) return 0;
@@ -786,7 +667,7 @@ int ctn_pw_tma(const PwArgs& a, int pro, int epi, cudaStream_t st) {
   TmaArgs g;
   memset(&g, 0, sizeof(g));
   g.a = a;
-  g.n_tile = a.M >= 256 ? 256 : ((a.M + 15) / 16) * 16;
+  g.n_tile = pick_n_tile(a.M);
   g.n_tiles = (a.M + g.n_tile - 1) / g.n_tile;
   g.k_slabs = (a.K + KS - 1) / KS;
   g.t_tiles = a.pitch / TM;
@@ -796,21 +677,13 @@ int ctn_pw_tma(const PwArgs& a, int pro, int epi, cudaStream_t st) {
   g.oscale = reinterpret_cast<const float*>(g.wimg + (size_t)g.n_tiles * g.k_slabs * 2 * g.n_tile * KS * sizeof(__half));
   g.act_scale = a.act_scale;
   g.dwp = a.dw_params;
-  // CTA pairs (opt-in with CTN_TMA_PAIR=1; N/2 rows of W per CTA must be a multiple of 16).  Parity-green, but measured SLOWER on cfg2
-  // (step 7.52 vs 6.62 ms, pw2 3.61 vs 3.06 ms, gpurun call L): the per-slab relay of the peer's "stage full" to the leader and the
-  // lock-step of two CTAs cost more than the halved weight traffic buys -- the single-CTA form stays the default.
-  static const char* env_pair = getenv("CTN_TMA_PAIR");
-  g.pair = (env_pair ? atoi(env_pair) != 0 : 0) && g.n_tile % 32 == 0 && g.n_tile >= 64 && a.B * g.t_tiles >= 2 && num_sms() >= 2;
-  g.idesc = ptx::make_idesc_f16(g.pair ? 2 * TM : TM, g.n_tile, /*A MN-major*/ 1, /*B K-major*/ 0);
-  static const char* env_dbg = getenv("CTN_UMMA_DBG");
-  g.dbg = env_dbg ? (uint32_t)atoi(env_dbg) : 0u;
+  g.idesc = ptx::make_idesc_f16(TM, g.n_tile, /*A MN-major*/ 1, /*B K-major*/ 0);
   // header: barriers + epilogue parameters (HDR_FIXED), the output scale table, then (PRO_RES) the folded bias vectors v1, v2 of the
   // previous block for all K channels (two global loads per channel and stage sat on the producers' critical path otherwise)
   g.res_tab_off = (uint32_t)(HDR_FIXED + g.n_tiles * g.n_tile * 4);
-  static const char* env_rev = getenv("CTN_TMA_REVERSE");
-  g.reverse = (pro == PRO_DW) && (env_rev ? atoi(env_rev) != 0 : 1);
+  g.reverse = pro == PRO_DW;
   g.hdr_bytes = (uint32_t)((g.res_tab_off + (pro == PRO_RES ? 2 * g.k_slabs * KS * 4 : 0) + 1023) & ~1023u);
-  g.op_stage_bytes = 2u * A_BYTES + (g.pair ? 1u : 2u) * g.w_bytes;
+  g.op_stage_bytes = 2u * A_BYTES + 2u * g.w_bytes;
   uint32_t raw_data = 0;
   if (pro == PRO_DW) {
     const int d = a.dw_dilation;
@@ -828,28 +701,17 @@ int ctn_pw_tma(const PwArgs& a, int pro, int epi, cudaStream_t st) {
   g.raw_stage_bytes = (g.raw_tx_bytes + 1023u) & ~1023u;
   const size_t dec_bytes = epi == EPI_MASKDEC ? ((size_t)a.Nb * 16 + 2 * 128 * 16) * sizeof(float) : 0;
   const size_t budget = 227 * 1024 - 1024 - g.hdr_bytes - dec_bytes;
-  static const char* env_ops = getenv("CTN_TMA_OPSTAGES");
-  int op = env_ops ? atoi(env_ops) : (g.pair ? 4 : 3);
-  if (op < 2) op = 2;
-  if (op > MAX_OP) op = MAX_OP;
+  // 3 operand stages (fewer if they do not fit), then as many raw stages as fit
+  int op = 3;
   while (op > 2 && (size_t)op * g.op_stage_bytes + 2 * (size_t)g.raw_stage_bytes > budget) --op;
   if ((size_t)op * g.op_stage_bytes + 2 * (size_t)g.raw_stage_bytes > budget) return CTN_EUNSUPPORTED;
   int raw = (int)((budget - (size_t)op * g.op_stage_bytes) / g.raw_stage_bytes);
   if (raw > MAX_RAW) raw = MAX_RAW;
-  static const char* env_raw = getenv("CTN_TMA_RAWSTAGES");
-  if (env_raw && atoi(env_raw) >= 2 && atoi(env_raw) < raw) raw = atoi(env_raw);
   g.op_stages = op;
   g.raw_stages = raw;
   const size_t smem = 1024 + g.hdr_bytes + (size_t)op * g.op_stage_bytes + (size_t)raw * g.raw_stage_bytes + dec_bytes;
-  int grid = num_sms();
-  static const char* env_grid = getenv("CTN_UMMA_GRID");
-  if (env_grid && atoi(env_grid) > 0) grid = atoi(env_grid);
-  if (g.pair) {
-    const int groups = (a.B * g.t_tiles + 1) / 2;
-    const int cl_items = epi == EPI_MASKDEC ? groups : groups * g.n_tiles;
-    grid &= ~1;
-    if (grid > 2 * cl_items) grid = 2 * cl_items;
-  } else if (grid > g.num_items) grid = g.num_items;
+  int grid = ctn_num_sms();
+  if (grid > g.num_items) grid = g.num_items;
   if (pro == PRO_DW && epi == EPI_RAW) {
     if (a.dw_in_slope) {  // training forward
       if (g.dw_three) return launch<PRO_DW, EPI_RAW, 8 | 4>(g, smem, grid, st);
@@ -864,7 +726,7 @@ int ctn_pw_tma(const PwArgs& a, int pro, int epi, cudaStream_t st) {
   if (pro == PRO_NONE && epi == EPI_H) return launch<PRO_NONE, EPI_H>(g, smem, grid, st);
   if (pro == PRO_PRELU && epi == EPI_MASKDEC) {
     const int tiles = a.B * g.t_tiles;
-    return launch<PRO_PRELU, EPI_MASKDEC>(g, smem, (g.pair || grid < tiles) ? grid : tiles, st);
+    return launch<PRO_PRELU, EPI_MASKDEC>(g, smem, grid < tiles ? grid : tiles, st);
   }
   return CTN_EUNSUPPORTED;
 }

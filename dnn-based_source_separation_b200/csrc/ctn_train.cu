@@ -799,8 +799,7 @@ int transpose(const float* W, float* Wt, int M, int K, cudaStream_t st) {
 // configured mode is plain fp32, where the FFMA split-K kernel runs.
 int wgrad(const ctn_config_t* c, const float* dy, size_t dy_bs, const float* x, size_t x_bs, float* dWa, float* dWb, int split_row,
           int M, int K, int B, int frames, int pitch, cudaStream_t st) {
-  static const char* env = getenv("CTN_WGRAD_SIMT");  // debug: force the FFMA kernel
-  if (c->math != CTN_MATH_FP32 && !(env && atoi(env)))
+  if (c->math != CTN_MATH_FP32)
     return ctn_wgrad_umma(dy, dy_bs, x, x_bs, dWa, dWb, split_row, M, K, B, frames, pitch, c->math, st);
   const int parts = dWb ? 2 : 1;
   for (int part = 0; part < parts; ++part) {
@@ -917,8 +916,7 @@ extern "C" int ctn_convtasnet_fwd_train(const ctn_config_t* c, const ctn_params_
   // pre-activation behind for the backward -- 2 launches per block instead of 7, no u / gLN2(u) round trips
   bool fused = false;
   const float* mask_scale = nullptr;
-  static const char* env_unf = getenv("CTN_TRAIN_UNFUSED");
-  if (ws.tcn_mem && !(env_unf && atoi(env_unf))) {
+  if (ws.tcn_mem) {
     TcnTrainHooks hk{ws.x.data(), ws.hpre.data(), ws.upre.data()};
     const int rc = ctn_tcn_train_fwd(c, p->blocks, ws.tcn_mem, ws.tcn_bytes, &hk, ws.stats, ws.skip, ws.head.vb, Bc, p->prelu_out, &mask_scale,
                                      B, frames, pitch, st);

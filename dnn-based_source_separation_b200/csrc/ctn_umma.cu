@@ -24,8 +24,6 @@
 #include "ctn_umma_ptx.cuh"
 #include "ctn_dw_math.cuh"
 #include <cuda_fp16.h>
-#include <stdlib.h>
-#include <string.h>
 
 namespace {
 
@@ -41,10 +39,8 @@ constexpr uint32_t W_LAYOUT = KS == 32 ? 2u : 4u;    // UMMA layout type of the 
 constexpr uint32_t W_SBO = KS == 32 ? 1024u : 512u;  // bytes between 8-row groups of the weight image
 constexpr int NUM_THREADS_DW = 21 * 32;   // PRO_DW kernels: 4 epilogue + 1 MMA + 16 producer warps (2 channels each)
 constexpr int NUM_THREADS_E8 = 17 * 32;   // other kernels: 4 + 1 + 8 producer warps + a second epilogue warpgroup (13-16)
-constexpr int NUM_THREADS_RES = 25 * 32;  // PRO_RES kernels (CTN_RES_WARPS16): 4 + 1 + 16 producer warps + second epilogue warpgroup (21-24)
-constexpr int F16_MAX_ROWS = 2048;  // fp16-piece mode: padded output channels whose scales fit the shared-memory table
-constexpr int SMEM_HEADER = 2048 + F16_MAX_ROWS * 4;  // barriers + tmem pointer, the epilogue parameter row, the fp16-mode output scales
-constexpr int SMEM_SCALES = 2048;   // byte offset of float[F16_MAX_ROWS]: power-of-two scale of every padded output channel of the
+constexpr int SMEM_HEADER = 2048 + CTN_F16_MAX_ROWS * 4;  // barriers + tmem pointer, the epilogue parameter row, the fp16-mode output scales
+constexpr int SMEM_SCALES = 2048;   // byte offset of float[CTN_F16_MAX_ROWS]: power-of-two scale of every padded output channel of the
                                     // contraction (F16 kernels), loaded ONCE per CTA (a per-item staging put a global-load latency
                                     // on the epilogue's critical path: +0.9 us per item, 0.5 ms per step)
 constexpr int SMEM_PARAMS = 1024;   // byte offset of float[256] inside the header
@@ -56,8 +52,6 @@ struct UmmaArgs {
   int n_tile, n_tiles, k_slabs, t_tiles, num_items, stages;
   uint32_t stage_bytes, w_bytes;  // w_bytes: bytes per precision of a weight slab (n_tile*128)
   uint32_t idesc, lbo_a, sbo_a, lbo_w, sbo_w, a_layout, w_layout;
-  int cluster, tiles_total, cluster_items, wsplit;  // 2 = CTA pair (cta_group::2 MMA, each CTA stages half of the weight slab); B*t_tiles; n_tiles*ceil(tiles/cluster)
-  uint32_t dbg;  // CTN_UMMA_DBG bits: 1 = no epilogue stores, 2 = no activation loads, 4 = no weight copies, 8 = no MMA
 };
 
 // producer warps per prologue: the depthwise producer always runs 16; the residual-update producer (pw1, the second
@@ -72,14 +66,6 @@ template <int PRO> struct Roles {
 };
 static_assert(Roles<PRO_DW>::THREADS == NUM_THREADS_DW && Roles<PRO_NONE>::THREADS == NUM_THREADS_E8, "role layout");
 
-// debug timeline (CTN_UMMA_DBG bit 128): CTA 0 records globaltimer stamps per role and slab
-__device__ unsigned long long g_timeline[3 * 4096];
-__device__ __forceinline__ unsigned long long gtime() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-
 struct __align__(8) SmemHeader {
   uint64_t full[MAX_STAGES];
   uint64_t empty[MAX_STAGES];
@@ -89,7 +75,7 @@ struct __align__(8) SmemHeader {
 };
 
 template <int DCLS, bool INTERIOR, int CPW>
-__device__ __forceinline__ void dw_slab(const PwArgs& a, int b, int ks, int pw, int tbase, float2 mr1, float pslope, bool skip_loads,
+__device__ __forceinline__ void dw_slab(const PwArgs& a, int b, int ks, int pw, int tbase, float2 mr1, float pslope,
                                         bool prefetch_next, float4 (&v)[CPW], float2& dls, float2& dlss) {
   const int d = a.dw_dilation, pl = a.dw_pad_left;
   const int step = DCLS == 4 ? d : 4;
@@ -105,7 +91,7 @@ __device__ __forceinline__ void dw_slab(const PwArgs& a, int b, int ks, int pw, 
     for (int k = 0; k < 3; ++k) {
       int ts = first + k * step;
       if (!INTERIOR) ts = ts < 0 ? 0 : (ts > a.pitch - 4 ? a.pitch - 4 : ts);
-      q[j][k] = skip_loads ? make_float4(1.f, 2.f, 3.f, 4.f) : __ldg(reinterpret_cast<const float4*>(hr + ts));
+      q[j][k] = __ldg(reinterpret_cast<const float4*>(hr + ts));
     }
     pg[j] = __ldg(a.dw_norm_g + cc); pb[j] = __ldg(a.dw_norm_b + cc); pbd[j] = __ldg(a.dw_b + cc);
     pw0[j] = __ldg(a.dw_w + cc * 3); pw1[j] = __ldg(a.dw_w + cc * 3 + 1); pw2[j] = __ldg(a.dw_w + cc * 3 + 2);
@@ -128,16 +114,14 @@ __device__ __forceinline__ void dw_slab(const PwArgs& a, int b, int ks, int pw, 
   }
 }
 
-// PAIR: the kernel runs as clusters of 2 CTAs driving cta_group::2 MMAs.  It is a template parameter (not a run-time
-// flag) because a kernel that contains cta_group::2 instructions can only be launched with an even cluster size.
 // F16: operands are staged as fp16 hi/lo pieces (kind::f16, "3xFP16"): A MN-major SWIZZLE_128B (atoms of 64 time steps x 8
 // channels), W K-major SWIZZLE_64B (rows of 32 channels = 64 bytes) -- both pinned on hardware by tools/umma_unit_f16.cu.
 // Half the shared-memory bytes per stage (4-deep ring at N = 256) and half the tensor-pipe time of the TF32 split.
-template <int PRO, int EPI, int NPASS, bool PAIR, bool F16>
+template <int PRO, int EPI, int NPASS, bool F16>
 __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_umma(const UmmaArgs g) {
   constexpr int NPREC = NPASS == 3 ? 2 : 1;  // precisions staged per operand (hi [, lo])
   constexpr int A_BYTES = F16 ? TM * KS * 2 : TM * KS * 4;  // bytes of one precision of the activation slab (shadows the tf32 constant)
-  static_assert(!F16 || (NPASS == 3 && !PAIR), "fp16 operands: 3-pass split, single-CTA only");
+  static_assert(!F16 || NPASS == 3, "fp16 operands: 3-pass split");
   constexpr int EGROUPS = Roles<PRO>::EGROUPS;  // epilogue warpgroups (each covers all 128 TMEM lanes)
   constexpr int PROD_WARPS = Roles<PRO>::PROD_WARPS;
   constexpr int CPW = KS / PROD_WARPS;            // channels of a slab per producer warp (2 or 4)
@@ -149,24 +133,19 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_umma(const UmmaAr
   const uint32_t stage0 = base + SMEM_HEADER;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const PwArgs& a = g.a;
-  constexpr bool pair = PAIR;  // CTA pair: cta_group::2 MMA (M = 256), each CTA stages its time tile and HALF of the weights
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < g.stages; ++s) {
-      // pair mode: the peer's producers fill the PEER's full[s]; its relay warp forwards one arrival to the leader's
-      ptx::mbar_init(ptx::smem_u32(&hdr->full[s]), PROD_WARPS + 1 + ((pair && ptx::cluster_ctarank() == 0) ? 1 : 0));
+      ptx::mbar_init(ptx::smem_u32(&hdr->full[s]), PROD_WARPS + 1);
       ptx::mbar_init(ptx::smem_u32(&hdr->empty[s]), 1);
     }
     for (int i = 0; i < 2; ++i) {
       ptx::mbar_init(ptx::smem_u32(&hdr->tfull[i]), 1);
-      ptx::mbar_init(ptx::smem_u32(&hdr->tempty[i]), pair ? 2 * 4 * EGROUPS : 128 * EGROUPS);
+      ptx::mbar_init(ptx::smem_u32(&hdr->tempty[i]), 128 * EGROUPS);
     }
     ptx::fence_mbar_init();
   }
-  if (warp == 4) {
-    if constexpr (pair) ptx::tmem_alloc2(ptx::smem_u32(&hdr->tmem_base), 512);
-    else ptx::tmem_alloc(ptx::smem_u32(&hdr->tmem_base), 512);
-  }
+  if (warp == 4) ptx::tmem_alloc(ptx::smem_u32(&hdr->tmem_base), 512);
   // fp16 pieces: power-of-two scale of the activation operand (|operand| * act_s <= 2^15 by construction, ctn_act_scales),
   // undone together with the weight-group scales in the epilogue
   float act_s = 1.f;
@@ -180,23 +159,16 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_umma(const UmmaAr
   __syncthreads();
   ptx::tc_fence_after();
   const uint32_t tmem_base = hdr->tmem_base;
-  if (pair) ptx::cluster_sync_all();  // barriers of every CTA initialised before any remote arrive / multicast
 
-  // Work decomposition.  A cluster of C CTAs walks the same sequence of cluster items J = cidx + it * num_clusters;
-  // J -> (weight tile nt = J % n_tiles, tile group J / n_tiles); CTA rank r of the cluster takes time tile
-  // L = group * C + r -> (b, tt).  All CTAs of a cluster therefore need the SAME weight slabs at the same step, of which
-  // each CTA of a pair stages one half; ranks whose L falls off the end run a dummy item (no loads, no stores).
-  const int crank = pair ? (int)ptx::cluster_ctarank() : 0;
-  const int cidx = (int)blockIdx.x / g.cluster, num_clusters = (int)gridDim.x / g.cluster;
-  const int items_per_cta = (g.cluster_items - cidx + num_clusters - 1) / num_clusters;
-  auto decode = [&](int it2, int& nt2, int& tt2, int& b2) -> bool {
-    const int J = cidx + it2 * num_clusters;
+  // Work decomposition: CTA c walks the items J = c + it * gridDim.x; J -> (weight tile nt = J % n_tiles, time tile
+  // L = J / n_tiles -> (b, tt)).  n-tile fastest: co-running CTAs read the same activations while they are in L2.
+  const int items_per_cta = (g.num_items - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
+  auto decode = [&](int it2, int& nt2, int& tt2, int& b2) {
+    const int J = (int)blockIdx.x + it2 * (int)gridDim.x;
     nt2 = J % g.n_tiles;
-    const int L = (J / g.n_tiles) * g.cluster + crank;
+    const int L = J / g.n_tiles;
     tt2 = L % g.t_tiles;
     b2 = L / g.t_tiles;
-    if (L >= g.tiles_total) { tt2 = 0; b2 = 0; return false; }
-    return true;
   };
 
   if (warp >= 5 && warp < 5 + PROD_WARPS) {
@@ -211,20 +183,19 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_umma(const UmmaAr
     // boundaries, so that the global-load latency overlaps the split/store work and the barrier waits
     auto load_A = [&](int it2, int ks2, float4 (&dst)[CPW], float4 (&dstr)[CPW]) {
       int nt2, tt2, b2;
-      const bool live2 = decode(it2, nt2, tt2, b2);
+      decode(it2, nt2, tt2, b2);
       const float* Ab2 = a.A + (size_t)b2 * a.K * a.pitch + (size_t)tt2 * TM + lane * 4;
 #pragma unroll
       for (int j = 0; j < CPW; ++j) {
         const int k = ks2 * KS + pw * CPW + j;
-        dst[j] = (k < a.K && live2 && !(g.dbg & 2u)) ? __ldg(reinterpret_cast<const float4*>(Ab2 + (size_t)k * a.pitch))
-                                             : make_float4(0.f, 0.f, 0.f, 0.f);
+        dst[j] = k < a.K ? __ldg(reinterpret_cast<const float4*>(Ab2 + (size_t)k * a.pitch)) : make_float4(0.f, 0.f, 0.f, 0.f);
       }
       if (PRO == PRO_RES) {
         const float* Rb2 = a.res_r + (size_t)b2 * a.res_Mt * a.pitch + (size_t)tt2 * TM + lane * 4;
 #pragma unroll
         for (int j = 0; j < CPW; ++j) {
           const int k = ks2 * KS + pw * CPW + j;
-          dstr[j] = (k < a.K && live2) ? __ldg(reinterpret_cast<const float4*>(Rb2 + (size_t)k * a.pitch)) : make_float4(0.f, 0.f, 0.f, 0.f);
+          dstr[j] = k < a.K ? __ldg(reinterpret_cast<const float4*>(Rb2 + (size_t)k * a.pitch)) : make_float4(0.f, 0.f, 0.f, 0.f);
         }
       }
     };
@@ -232,7 +203,7 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_umma(const UmmaAr
     if (PRO != PRO_DW && items_per_cta > 0) load_A(0, 0, vnext, rnext);
     for (int it = 0; it < items_per_cta; ++it) {
       int nt, tt, b;
-      const bool live = decode(it, nt, tt, b);
+      decode(it, nt, tt, b);
       const uint8_t* wsrc = reinterpret_cast<const uint8_t*>(g.wimg) + (size_t)nt * g.k_slabs * NPREC * g.w_bytes;
       // PRO_DW: per-sample gLN1 statistics of h (the A operand)
       float2 mr1 = make_float2(0.f, 1.f);
@@ -270,9 +241,9 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_umma(const UmmaAr
               if (tbase + 1 >= a.frames) xn.y = 0.f;
               if (tbase + 2 >= a.frames) xn.z = 0.f;
               if (tbase + 3 >= a.frames) xn.w = 0.f;
-              if (k >= a.K || !live) xn = make_float4(0.f, 0.f, 0.f, 0.f);
+              if (k >= a.K) xn = make_float4(0.f, 0.f, 0.f, 0.f);
               v[j] = xn;
-              if (nt == 0 && live && k < a.K)
+              if (nt == 0 && k < a.K)
                 *reinterpret_cast<float4*>(a.res_x_out + ((size_t)b * a.K + k) * a.pitch + tbase) = xn;
             }
           }
@@ -283,49 +254,26 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_umma(const UmmaAr
           // u[c][t] = PReLU( sum_k wd[c][k] * hn[c][t + k*d - pl] + bd[c] ), hn = gLN1(h) inside [0,frames), 0 outside.
           // All 12 128-bit loads of the slab (4 channels x 3 taps) are issued before any arithmetic.  The branch below is
           // uniform over the CTA (depends on the item only).
-          const bool skipl = (g.dbg & 2u) != 0;
-          const bool pfn = (ks + 1 < g.k_slabs) && !(g.dbg & 16u);
-          if (!live) {
-#pragma unroll
-            for (int j = 0; j < CPW; ++j) v[j] = make_float4(0.f, 0.f, 0.f, 0.f);
-          } else if (dw_interior) {
-            if (dcls == 4) dw_slab<4, true, CPW>(a, b, ks, pw, tbase, mr1, pslope, skipl, pfn, v, dls, dlss);
-            else if (dcls == 2) dw_slab<2, true, CPW>(a, b, ks, pw, tbase, mr1, pslope, skipl, pfn, v, dls, dlss);
-            else dw_slab<1, true, CPW>(a, b, ks, pw, tbase, mr1, pslope, skipl, pfn, v, dls, dlss);
+          const bool pfn = ks + 1 < g.k_slabs;
+          if (dw_interior) {
+            if (dcls == 4) dw_slab<4, true, CPW>(a, b, ks, pw, tbase, mr1, pslope, pfn, v, dls, dlss);
+            else if (dcls == 2) dw_slab<2, true, CPW>(a, b, ks, pw, tbase, mr1, pslope, pfn, v, dls, dlss);
+            else dw_slab<1, true, CPW>(a, b, ks, pw, tbase, mr1, pslope, pfn, v, dls, dlss);
           } else {
-            if (dcls == 4) dw_slab<4, false, CPW>(a, b, ks, pw, tbase, mr1, pslope, skipl, pfn, v, dls, dlss);
-            else if (dcls == 2) dw_slab<2, false, CPW>(a, b, ks, pw, tbase, mr1, pslope, skipl, pfn, v, dls, dlss);
-            else dw_slab<1, false, CPW>(a, b, ks, pw, tbase, mr1, pslope, skipl, pfn, v, dls, dlss);
+            if (dcls == 4) dw_slab<4, false, CPW>(a, b, ks, pw, tbase, mr1, pslope, pfn, v, dls, dlss);
+            else if (dcls == 2) dw_slab<2, false, CPW>(a, b, ks, pw, tbase, mr1, pslope, pfn, v, dls, dlss);
+            else dw_slab<1, false, CPW>(a, b, ks, pw, tbase, mr1, pslope, pfn, v, dls, dlss);
           }
         }
-        const bool tl = (g.dbg & 128u) && blockIdx.x == 0 && p == 0 && (it * g.k_slabs + ks) < 1024;
-        if (tl) g_timeline[(it * g.k_slabs + ks) * 4 + 0] = gtime();
         ptx::mbar_wait(ptx::smem_u32(&hdr->empty[s]), ph ^ 1u);
-        if (tl) g_timeline[(it * g.k_slabs + ks) * 4 + 1] = gtime();
         const uint32_t st_base = stage0 + (uint32_t)s * g.stage_bytes;
         if (p == 0) {
           const uint32_t fb = ptx::smem_u32(&hdr->full[s]);
-          if (g.dbg & 4u) {
-            ptx::mbar_arrive(fb);
-          } else if (!pair) {
-            ptx::mbar_arrive_expect_tx(fb, NPREC * g.w_bytes);
-            const uint32_t chunk = NPREC * g.w_bytes / (uint32_t)g.wsplit;  // several requests in flight per slab
-            for (int c = 0; c < g.wsplit; ++c)
-              ptx::bulk_g2s(st_base + NPREC * A_BYTES + c * chunk, wsrc + (size_t)ks * NPREC * g.w_bytes + (size_t)c * chunk, chunk, fb);
-          } else {
-            // pair mode: this CTA stages rows [crank*n_tile/2, +n_tile/2) of the slab (a contiguous half of the hi image and
-            // of the lo image); the copy completes on this CTA's own full[s].
-            const uint32_t half = g.w_bytes / 2;
-            const uint32_t lb = fb;
-            ptx::mbar_arrive_expect_tx(lb, NPREC * half);
-            const uint8_t* src = wsrc + (size_t)ks * NPREC * g.w_bytes + (size_t)crank * half;
-#pragma unroll
-            for (int pr = 0; pr < NPREC; ++pr)
-              ptx::bulk_g2s(st_base + NPREC * A_BYTES + pr * half, src + (size_t)pr * g.w_bytes, half, lb);
-          }
+          ptx::mbar_arrive_expect_tx(fb, NPREC * g.w_bytes);
+          ptx::bulk_g2s(st_base + NPREC * A_BYTES, wsrc + (size_t)ks * NPREC * g.w_bytes, NPREC * g.w_bytes, fb);
         }
 #pragma unroll
-        for (int j = 0; j < ((g.dbg & 64u) ? 0 : CPW); ++j) {
+        for (int j = 0; j < CPW; ++j) {
           const int kl = pw * CPW + j;  // 0..KS-1 within the slab
           const int kg = kl >> 2, r = kl & 3;
           // MN-major tf32 needs SWIZZLE_128B_BASE32B (the only MN-major layout the tensor core accepts for 32-bit
@@ -364,10 +312,9 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_umma(const UmmaAr
         ptx::fence_proxy_async_smem();
         __syncwarp();
         if (lane == 0) ptx::mbar_arrive(ptx::smem_u32(&hdr->full[s]));
-        if (tl) g_timeline[(it * g.k_slabs + ks) * 4 + 2] = gtime();
         if (++s == g.stages) { s = 0; ph ^= 1u; }
       }
-      if (PRO == PRO_DW && nt == 0 && live) {
+      if (PRO == PRO_DW && nt == 0) {
         const double sd = warp_sum_d((double)dls.x + (double)dls.y), ssd = warp_sum_d((double)dlss.x + (double)dlss.y);
         if (lane == 0) { atomicAdd(&a.dw_stats_out[2 * b], sd); atomicAdd(&a.dw_stats_out[2 * b + 1], ssd); }
       }
@@ -377,81 +324,51 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_umma(const UmmaAr
     // The whole warp walks the loop converged; one elected lane issues.  The stage-free commit of slab q is issued
     // AFTER the first MMA of slab q+1 (same item), so the tensor pipe always has work queued while the thread is busy
     // with the commit / barrier bookkeeping.
-    if (!pair || crank == 0) {  // pair mode: only the leader CTA issues (its MMAs span both CTAs' TMEM and smem)
-      int s = 0;
-      uint32_t ph = 0;
-      const bool leader = ptx::elect_one();
-      const uint32_t w_lo_off = (pair ? g.w_bytes / 2 : g.w_bytes) >> 4;
-      // descriptor templates: only the 14-bit start-address field changes
-      const uint64_t da_t = ptx::make_smem_desc(0, g.lbo_a, g.sbo_a, g.a_layout);
-      const uint64_t dw_t = ptx::make_smem_desc(0, g.lbo_w, g.sbo_w, g.w_layout);
-      for (int it = 0; it < items_per_cta; ++it) {
-        const int acc = it & 1;
-        if (pair) ptx::mbar_wait_cluster(ptx::smem_u32(&hdr->tempty[acc]), ((uint32_t)(it >> 1) & 1u) ^ 1u);
-        else ptx::mbar_wait(ptx::smem_u32(&hdr->tempty[acc]), ((uint32_t)(it >> 1) & 1u) ^ 1u);
+    int s = 0;
+    uint32_t ph = 0;
+    const bool leader = ptx::elect_one();
+    // descriptor templates: only the 14-bit start-address field changes
+    const uint64_t da_t = ptx::make_smem_desc(0, g.lbo_a, g.sbo_a, g.a_layout);
+    const uint64_t dw_t = ptx::make_smem_desc(0, g.lbo_w, g.sbo_w, g.w_layout);
+    for (int it = 0; it < items_per_cta; ++it) {
+      const int acc = it & 1;
+      ptx::mbar_wait(ptx::smem_u32(&hdr->tempty[acc]), ((uint32_t)(it >> 1) & 1u) ^ 1u);
+      ptx::tc_fence_after();
+      const uint32_t d_tmem = tmem_base + (uint32_t)acc * 256u;
+      int prev_s = -1;
+      for (int ks = 0; ks < g.k_slabs; ++ks) {
+        ptx::mbar_wait(ptx::smem_u32(&hdr->full[s]), ph);
         ptx::tc_fence_after();
-        const uint32_t d_tmem = tmem_base + (uint32_t)acc * 256u;
-        int prev_s = -1;
-        for (int ks = 0; ks < g.k_slabs; ++ks) {
-          const bool tl = (g.dbg & 128u) && blockIdx.x == 0 && lane == 0 && (it * g.k_slabs + ks) < 1024;
-          if (tl) g_timeline[4096 + (it * g.k_slabs + ks) * 4 + 0] = gtime();
-          if (pair) ptx::mbar_wait_cluster(ptx::smem_u32(&hdr->full[s]), ph);
-          else ptx::mbar_wait(ptx::smem_u32(&hdr->full[s]), ph);
-          if (tl) g_timeline[4096 + (it * g.k_slabs + ks) * 4 + 1] = gtime();
-          ptx::tc_fence_after();
-          const uint32_t st_base = stage0 + (uint32_t)s * g.stage_bytes;
-          const uint32_t a_hi = st_base >> 4, a_lo = (st_base + A_BYTES) >> 4;
-          const uint32_t w_hi = (st_base + NPREC * A_BYTES) >> 4, w_lo = w_hi + w_lo_off;
-          if (leader) {
-            auto commit = [&](uint64_t* bar) {
-              if constexpr (pair) ptx::mma2_commit_multicast(ptx::smem_u32(bar), (uint16_t)3u);  // same barrier in both CTAs
-              else ptx::mma_commit(ptx::smem_u32(bar));
-            };
-            auto mma = [&](uint64_t da, uint64_t dw, uint32_t accum) {
-              if constexpr (pair) ptx::mma2_tf32(d_tmem, da, dw, g.idesc, accum);
-              else if constexpr (F16) ptx::mma_f16(d_tmem, da, dw, g.idesc, accum);
-              else ptx::mma_tf32(d_tmem, da, dw, g.idesc, accum);
-            };
+        const uint32_t st_base = stage0 + (uint32_t)s * g.stage_bytes;
+        const uint32_t a_hi = st_base >> 4, a_lo = (st_base + A_BYTES) >> 4;
+        const uint32_t w_hi = (st_base + NPREC * A_BYTES) >> 4, w_lo = w_hi + (g.w_bytes >> 4);
+        if (leader) {
+          auto mma = [&](uint64_t da, uint64_t dw, uint32_t accum) {
+            if constexpr (F16) ptx::mma_f16(d_tmem, da, dw, g.idesc, accum);
+            else ptx::mma_tf32(d_tmem, da, dw, g.idesc, accum);
+          };
 #pragma unroll
-            // per instruction: 8 channels (tf32) or 16 (fp16); either way the A start address advances by 4096 B (two channel
-            // groups) and the W start address by 32 B
-            for (int kk = 0; kk < (F16 ? KS / 16 : KS / 8); ++kk) {
-              if (g.dbg & 8u) break;
-              const uint64_t da_hi = da_t | (uint64_t)(a_hi + kk * 256), dw_hi = dw_t | (uint64_t)(w_hi + kk * 2);
-              mma(da_hi, dw_hi, (ks | kk) ? 1u : 0u);
-              if (kk == 0 && prev_s >= 0) commit(&hdr->empty[prev_s]);  // previous slab's stage (its MMAs are queued ahead)
-              if (NPASS == 3) {
-                const uint64_t da_lo = da_t | (uint64_t)(a_lo + kk * 256), dw_lo = dw_t | (uint64_t)(w_lo + kk * 2);
-                mma(da_lo, dw_hi, 1u);
-                mma(da_hi, dw_lo, 1u);
-              }
-            }
-            if ((g.dbg & 8u) && prev_s >= 0) commit(&hdr->empty[prev_s]);
-            if (ks == g.k_slabs - 1) {
-              commit(&hdr->empty[s]);     // last slab of the item: free its stage right away
-              commit(&hdr->tfull[acc]);   // accumulator ready for the epilogue
+          // per instruction: 8 channels (tf32) or 16 (fp16); either way the A start address advances by 4096 B (two channel
+          // groups) and the W start address by 32 B
+          for (int kk = 0; kk < (F16 ? KS / 16 : KS / 8); ++kk) {
+            const uint64_t da_hi = da_t | (uint64_t)(a_hi + kk * 256), dw_hi = dw_t | (uint64_t)(w_hi + kk * 2);
+            mma(da_hi, dw_hi, (ks | kk) ? 1u : 0u);
+            if (kk == 0 && prev_s >= 0) ptx::mma_commit(ptx::smem_u32(&hdr->empty[prev_s]));  // previous slab's stage (its MMAs are queued ahead)
+            if (NPASS == 3) {
+              const uint64_t da_lo = da_t | (uint64_t)(a_lo + kk * 256), dw_lo = dw_t | (uint64_t)(w_lo + kk * 2);
+              mma(da_lo, dw_hi, 1u);
+              mma(da_hi, dw_lo, 1u);
             }
           }
-          __syncwarp();
-          if (tl) g_timeline[4096 + (it * g.k_slabs + ks) * 4 + 2] = gtime();
-          prev_s = s;
-          if (++s == g.stages) { s = 0; ph ^= 1u; }
+          if (ks == g.k_slabs - 1) {
+            ptx::mma_commit(ptx::smem_u32(&hdr->empty[s]));     // last slab of the item: free its stage right away
+            ptx::mma_commit(ptx::smem_u32(&hdr->tfull[acc]));   // accumulator ready for the epilogue
+          }
         }
+        __syncwarp();
+        prev_s = s;
+        if (++s == g.stages) { s = 0; ph ^= 1u; }
       }
-    }
-    else {
-      // peer CTA of a pair: this warp has no MMAs to issue; it forwards "my stage s is full" (the peer's local full[s]:
-      // its producer warps + its half of the weight slab) to the leader's full[s] with ONE cluster-scope arrival per
-      // slab, which keeps remote arrivals and cluster-scope releases off the producers' path
-      int s = 0;
-      uint32_t ph = 0;
-      for (int it = 0; it < items_per_cta; ++it)
-        for (int ks = 0; ks < g.k_slabs; ++ks) {
-          ptx::mbar_wait(ptx::smem_u32(&hdr->full[s]), ph);
-          if (lane == 0) ptx::mbar_arrive_remote(ptx::smem_u32(&hdr->full[s]), 0);
-          __syncwarp();
-          if (++s == g.stages) { s = 0; ph ^= 1u; }
-        }
     }
     __syncwarp();
   } else {
@@ -468,12 +385,12 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_umma(const UmmaAr
     const int tid_e = egroup * 128 + te;
     for (int it = 0; it < items_per_cta; ++it) {
       int nt, tt, b;
-      const bool live = decode(it, nt, tt, b);
+      decode(it, nt, tt, b);
       const int acc = it & 1;
       const int t = tt * TM + te;
       const bool tvalid = t < a.frames;
       const int n0 = nt * g.n_tile;
-      const int nvalid = live ? min(g.n_tile, a.M - n0) : 0;  // dummy item: nothing to read, store or count
+      const int nvalid = min(g.n_tile, a.M - n0);
       float mscale = 1.f;
       {
         // stage the per-channel parameter: EPI_HEAD: v1 - mean*rstd*v2 (deferred gLN shift); EPI_H / EPI_MASK: bias
@@ -490,10 +407,7 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_umma(const UmmaAr
         }
         asm volatile("bar.sync 1, %0;" ::"n"(128 * EGROUPS) : "memory");
       }
-      const bool tle = (g.dbg & 128u) && blockIdx.x == 0 && threadIdx.x == 0 && it < 1024;
-      if (tle) g_timeline[8192 + it * 4 + 0] = gtime();
       ptx::mbar_wait(ptx::smem_u32(&hdr->tfull[acc]), (uint32_t)(it >> 1) & 1u);
-      if (tle) g_timeline[8192 + it * 4 + 1] = gtime();
       ptx::tc_fence_after();
       const uint32_t taddr = tmem_base + (uint32_t)acc * 256u + ((uint32_t)((warp & 3) * 32) << 16);
       float* Dp = a.D + ((size_t)b * a.M + n0) * a.pitch + t;
@@ -506,7 +420,6 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_umma(const UmmaAr
       const int cbeg = egroup == 0 ? 0 : csplit;
       const int ncols = egroup == 0 ? csplit : ncols_all;
 
-      const bool do_store = !(g.dbg & 1u);
       const bool tile_full = tt * TM + TM <= a.frames;  // every time step of this tile is a real frame
       auto process = [&](const uint32_t (&buf)[16], int c0) {
         float wv[16];
@@ -520,7 +433,7 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_umma(const UmmaAr
         }
         float* q = Dp + (size_t)c0 * a.pitch;
         float* qm = Mp ? Mp + (size_t)c0 * a.pitch : nullptr;
-        const bool full = (c0 + 16 <= nvalid) && tile_full && do_store;  // warp-uniform
+        const bool full = (c0 + 16 <= nvalid) && tile_full;  // warp-uniform
         // F16: the 16 output channels of a chunk share one power-of-two weight scale (wimg_f16_rows scales 16-row groups)
         float osc = 1.f;
         if constexpr (F16) osc = reinterpret_cast<const float*>(smem + SMEM_SCALES)[n0 + c0];
@@ -573,10 +486,8 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_umma(const UmmaAr
           for (int j = 0; j < 16; ++j) {
             const float v = tvalid ? o[j] : 0.f;
             if (c0 + j < nvalid) {
-              if (do_store) {
-                q[(size_t)j * a.pitch] = v;
-                if (EPI == EPI_MASK && qm) qm[(size_t)j * a.pitch] = tvalid ? mk[j] : 0.f;
-              }
+              q[(size_t)j * a.pitch] = v;
+              if (EPI == EPI_MASK && qm) qm[(size_t)j * a.pitch] = tvalid ? mk[j] : 0.f;
               if (EPI == EPI_H) { const float sv = store_pre ? prelu_f(v, eslope) : v; ls += sv; lss = fmaf(sv, sv, lss); }
             }
           }
@@ -584,8 +495,8 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_umma(const UmmaAr
       };
 
       uint32_t bufA[16], bufB[16];
-      if (cbeg < ncols && !(g.dbg & 32u)) ptx::tmem_ld16(taddr + (uint32_t)cbeg, bufA);
-      for (int c0 = cbeg; c0 < ((g.dbg & 32u) ? 0 : ncols); c0 += 32) {
+      if (cbeg < ncols) ptx::tmem_ld16(taddr + (uint32_t)cbeg, bufA);
+      for (int c0 = cbeg; c0 < ncols; c0 += 32) {
         ptx::tmem_ld_wait();
         if (c0 + 16 < ncols) ptx::tmem_ld16(taddr + (uint32_t)(c0 + 16), bufB);
         process(bufA, c0);
@@ -594,16 +505,7 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_umma(const UmmaAr
         if (c0 + 16 < ncols) process(bufB, c0 + 16);
       }
       ptx::tc_fence_before();
-      if (pair) {  // one arrival per warp, on the LEADER's barrier (its MMA warp overwrites both CTAs' accumulators)
-        __syncwarp();
-        if (lane == 0) {
-          if (crank == 0) ptx::mbar_arrive(ptx::smem_u32(&hdr->tempty[acc]));
-          else ptx::mbar_arrive_remote(ptx::smem_u32(&hdr->tempty[acc]), 0);
-        }
-      } else {
-        ptx::mbar_arrive(ptx::smem_u32(&hdr->tempty[acc]));
-      }
-      if (tle) g_timeline[8192 + it * 4 + 2] = gtime();
+      ptx::mbar_arrive(ptx::smem_u32(&hdr->tempty[acc]));
       if (EPI == EPI_H) {
         double s = warp_sum_d((double)ls), ss = warp_sum_d((double)lss);
         if (lane == 0) { atomicAdd(&a.stats_out[2 * b], s); atomicAdd(&a.stats_out[2 * b + 1], ss); }
@@ -613,11 +515,7 @@ __global__ void __launch_bounds__(Roles<PRO>::THREADS, 1) k_pw_umma(const UmmaAr
   ptx::tc_fence_before();
   __syncthreads();
   ptx::tc_fence_after();
-  if (pair) ptx::cluster_sync_all();  // nobody exits while a peer may still multicast into it / arrive on it
-  if (warp == 4) {
-    if constexpr (pair) ptx::tmem_dealloc2(tmem_base, 512);
-    else ptx::tmem_dealloc(tmem_base, 512);
-  }
+  if (warp == 4) ptx::tmem_dealloc(tmem_base, 512);
 }
 
 // ---- weight images ---------------------------------------------------------------------------------------------
@@ -705,7 +603,7 @@ struct WimgJobs { WimgJob j[CTN_MAX_JOBS]; };
 // grid (max k_slabs * max n_tiles, jobs): one block per (slab, n-tile) of one job
 __global__ void __launch_bounds__(256) k_build_wimg_batch(const WimgJobs jobs, int nprec) {
   const WimgJob& jb = jobs.j[blockIdx.y];
-  const int n_tile = jb.M >= 256 ? 256 : ((jb.M + 15) / 16) * 16;
+  const int n_tile = pick_n_tile(jb.M);
   const int n_tiles = (jb.M + n_tile - 1) / n_tile, k_slabs = (jb.K + KS - 1) / KS;
   const size_t per = (size_t)n_tile * KS;
   for (int blk = blockIdx.x; blk < n_tiles * k_slabs; blk += gridDim.x) {
@@ -727,7 +625,7 @@ __global__ void __launch_bounds__(256) k_build_wimg_batch(const WimgJobs jobs, i
 __global__ void __launch_bounds__(512) k_build_wimg_batch_f16(const WimgJobs jobs) {
   __shared__ float smax[16];
   const WimgJob& jb = jobs.j[blockIdx.y];
-  const int n_tile = jb.M >= 256 ? 256 : ((jb.M + 15) / 16) * 16;
+  const int n_tile = pick_n_tile(jb.M);
   const int n_tiles = (jb.M + n_tile - 1) / n_tile, k_slabs = (jb.K + KS - 1) / KS;
   const int groups = n_tile / 16;
   __half* img = reinterpret_cast<__half*>(jb.wimg);
@@ -736,61 +634,16 @@ __global__ void __launch_bounds__(512) k_build_wimg_batch_f16(const WimgJobs job
     wimg_f16_group(jb.W, jb.M, jb.K, n_tile, k_slabs, blk / groups, blk % groups, img, oscale, smax);
 }
 
-int pick_n_tile(int M);
-// the fp16-piece mode keeps one scale per padded output channel in shared memory: contractions with more than
-// F16_MAX_ROWS padded output channels use the tf32 pieces instead (images and kernel are chosen by the same rule)
-int eff_math(int M, int math) {
-  if (math != CTN_MATH_F16X3) return math;
-  const int n_tile = pick_n_tile(M);
-  return ((M + n_tile - 1) / n_tile) * n_tile > F16_MAX_ROWS ? CTN_MATH_TF32X3 : math;
-}
-
-int pick_n_tile(int M) {
-  static const char* env_nt = getenv("CTN_UMMA_NTILE");
-  if (env_nt && atoi(env_nt) >= 16 && atoi(env_nt) <= 256 && atoi(env_nt) % 16 == 0 && M >= atoi(env_nt)) return atoi(env_nt);
-  if (M >= 256) return 256;
-  return ((M + 15) / 16) * 16;
-}
-
-int g_num_sms[CTN_MAX_DEVICES] = {0};  // per device ordinal
-int num_sms() {
-  const int dev = ctn_current_device();
-  if (g_num_sms[dev] == 0) {
-    cudaDeviceGetAttribute(&g_num_sms[dev], cudaDevAttrMultiProcessorCount, dev);
-    if (g_num_sms[dev] <= 0) g_num_sms[dev] = 148;
-  }
-  return g_num_sms[dev];
-}
-
-template <int PRO, int EPI, int NPASS, bool PAIR, bool F16>
+template <int PRO, int EPI, int NPASS, bool F16>
 int launch(const UmmaArgs& g, size_t smem, int grid, cudaStream_t st) {
-  constexpr int NT = Roles<PRO>::THREADS;
   static bool attr_done[CTN_MAX_DEVICES] = {false};  // the opt-in is per device (context)
   const int dev = ctn_current_device();
   if (!attr_done[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(k_pw_umma<PRO, EPI, NPASS, PAIR, F16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    cudaError_t e = cudaFuncSetAttribute(k_pw_umma<PRO, EPI, NPASS, F16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     if (e != cudaSuccess) return (int)e;
     attr_done[dev] = true;
   }
-  if (PAIR) {
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3(grid);
-    cfg.blockDim = dim3(NT);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, k_pw_umma<PRO, EPI, NPASS, PAIR, F16>, g);
-    if (e != cudaSuccess) return (int)e;
-  } else {
-    k_pw_umma<PRO, EPI, NPASS, PAIR, F16><<<grid, NT, smem, st>>>(g);
-  }
+  k_pw_umma<PRO, EPI, NPASS, F16><<<grid, Roles<PRO>::THREADS, smem, st>>>(g);
   CTN_COUNT_LAUNCH();
   CTN_RETURN_IF_CUDA_ERR();
   return CTN_OK;
@@ -799,13 +652,6 @@ int launch(const UmmaArgs& g, size_t smem, int grid, cudaStream_t st) {
 }  // namespace
 
 extern "C" int ctn_has_tcgen05(void) { return 1; }
-
-// debug: copy the timeline of the last CTN_UMMA_DBG&128 launch (3 regions x 4096 stamps) to the host
-extern "C" int ctn_debug_timeline(unsigned long long* host, int n) {
-  if (!host || n <= 0 || n > 3 * 4096) return CTN_EINVAL;
-  cudaError_t e = cudaMemcpyFromSymbol(host, g_timeline, sizeof(unsigned long long) * n);
-  return e == cudaSuccess ? CTN_OK : (int)e;
-}
 
 size_t ctn_umma_wimg_bytes(int M, int K, int math) {
   const int nprec = math == CTN_MATH_TF32 ? 1 : 2;
@@ -836,7 +682,7 @@ int ctn_umma_build_wimg_batch(const WimgJob* jobs, int n, int math, cudaStream_t
   const int nprec = math == CTN_MATH_TF32 ? 1 : 2;
   bool uniform = true;
   for (int i = 0; i < n; ++i) uniform = uniform && eff_math(jobs[i].M, math) == math;
-  if (getenv("CTN_UMMA_NTILE") || !uniform) {  // debug override changes the tiling: fall back to per-job launches
+  if (!uniform) {  // some jobs fall back to the tf32 pieces (eff_math): per-job launches
     for (int i = 0; i < n; ++i) CTN_TRY(ctn_umma_build_wimg(jobs[i].W, jobs[i].M, jobs[i].K, math, jobs[i].wimg, st));
     return CTN_OK;
   }
@@ -858,7 +704,6 @@ int ctn_umma_build_wimg_batch(const WimgJob* jobs, int n, int math, cudaStream_t
   return CTN_OK;
 }
 
-#define NPREC_HOST(m) ((m) == CTN_MATH_TF32 ? 1u : 2u)
 int ctn_pw_umma(const PwArgs& a, int pro, int epi, int math, cudaStream_t st) {
   if (!a.wimg) return CTN_EINVAL;
   math = eff_math(a.M, math);
@@ -876,32 +721,10 @@ int ctn_pw_umma(const PwArgs& a, int pro, int epi, int math, cudaStream_t st) {
   const bool f16 = math == CTN_MATH_F16X3;
   const uint32_t a_bytes = f16 ? (uint32_t)(TM * KS * 2) : (uint32_t)A_BYTES;
   g.w_bytes = (uint32_t)g.n_tile * (uint32_t)(KS * (f16 ? 2 : 4));
-  static const char* env_dbg = getenv("CTN_UMMA_DBG");
-  g.dbg = env_dbg ? (uint32_t)atoi(env_dbg) : 0u;
-  int grid = num_sms();
-  static const char* env_grid = getenv("CTN_UMMA_GRID");
-  if (env_grid && atoi(env_grid) > 0) grid = atoi(env_grid);
-  // CTA pairs (cluster of 2, tcgen05 cta_group::2; opt-in with CTN_UMMA_CLUSTER=2): one MMA covers two time tiles
-  // (M = 256) and each CTA stages only HALF of the weight slab, so a stage shrinks from 96 KB to 64 KB (3xTF32, n_tile
-  // 256) and the ring gets 3 stages instead of 2.  Parity-green on B200, but measured perf-neutral on cfg2 (10.59 vs
-  // 10.56 ms/step): with MMA-only (3.9 ms) and producer-only (4.2 ms) floors this close, the third stage does not buy
-  // overlap yet, so the simpler 1-CTA kernel stays the default (DESIGN.md section 6).
-  static const char* env_cl = getenv("CTN_UMMA_CLUSTER");
-  int cluster = env_cl ? atoi(env_cl) : 1;
-  if (cluster != 1 && cluster != 2) cluster = 1;
-  if (f16) cluster = 1;  // fp16 operands: single-CTA kernel only
-  g.tiles_total = a.B * g.t_tiles;
-  static const char* env_pm = getenv("CTN_UMMA_PAIR_MIN_N");
-  const int pair_min_n = env_pm ? atoi(env_pm) : 64;  // N = 64 / 256 are the pair shapes pinned by tools/umma_unit2.cu
-  if (cluster == 2 && (grid % 2 != 0 || g.tiles_total < 2 || g.n_tile % 32 != 0 || g.n_tile < pair_min_n)) cluster = 1;
-  g.cluster = cluster;
-  const uint32_t w_stage = cluster == 2 ? g.w_bytes / 2 : g.w_bytes;
-  g.stage_bytes = (uint32_t)nprec * (a_bytes + w_stage);
+  g.stage_bytes = (uint32_t)nprec * (a_bytes + g.w_bytes);
   const size_t budget = 227 * 1024 - SMEM_HEADER - 1024;
   int stages = (int)(budget / g.stage_bytes);
   if (stages > MAX_STAGES) stages = MAX_STAGES;
-  static const char* env_st = getenv("CTN_UMMA_STAGES");
-  if (env_st && atoi(env_st) >= 1 && atoi(env_st) < stages) stages = atoi(env_st);
   if (stages < 1) return CTN_EUNSUPPORTED;
   g.stages = stages;
   g.oscale = nullptr;
@@ -911,25 +734,20 @@ int ctn_pw_umma(const PwArgs& a, int pro, int epi, int math, cudaStream_t st) {
     g.lbo_a = 1024u; g.sbo_a = 2048u; g.a_layout = 2u;  // 64-time-step atoms adjacent, 8-channel groups 2048 B apart
     g.lbo_w = 16u; g.sbo_w = 512u; g.w_layout = 4u;      // SWIZZLE_64B rows of 32 k
   } else {
-    g.idesc = a.dbg_idesc ? a.dbg_idesc : ptx::make_idesc_tf32(cluster == 2 ? 2 * TM : TM, g.n_tile, /*A MN-major*/ 1, /*B K-major*/ 0);
-    g.lbo_a = a.dbg_lbo_a ? a.dbg_lbo_a : 512u;   // between 32-time-step atoms
-    g.sbo_a = a.dbg_sbo_a ? a.dbg_sbo_a : 2048u;  // between 4-channel groups
-    g.lbo_w = 16u;                                 // unused for swizzled K-major
-    g.sbo_w = a.dbg_sbo_w ? a.dbg_sbo_w : W_SBO;  // between 8-row (output channel) groups
+    g.idesc = ptx::make_idesc_tf32(TM, g.n_tile, /*A MN-major*/ 1, /*B K-major*/ 0);
+    g.lbo_a = 512u;   // between 32-time-step atoms
+    g.sbo_a = 2048u;  // between 4-channel groups
+    g.lbo_w = 16u;    // unused for swizzled K-major
+    g.sbo_w = W_SBO;  // between 8-row (output channel) groups
     g.a_layout = 1u; g.w_layout = W_LAYOUT;
   }
   const size_t smem = SMEM_HEADER + 1024 + (size_t)stages * g.stage_bytes;
-  static const char* env_ws = getenv("CTN_UMMA_WSPLIT");
-  g.wsplit = env_ws ? atoi(env_ws) : 1;
-  if (g.wsplit < 1 || g.wsplit > 16 || ((NPREC_HOST(math) * g.w_bytes / g.wsplit) % 16) != 0) g.wsplit = 1;
-  g.cluster_items = g.n_tiles * ((g.tiles_total + cluster - 1) / cluster);
-  const int max_grid = g.cluster_items * cluster;
-  if (grid > max_grid) grid = max_grid;
-#define UM_LAUNCH(P, E)                                                                   \
-  if (pro == P && epi == E)                                                               \
-    return f16 ? launch<P, E, 3, false, true>(g, smem, grid, st)                                                                  \
-           : nprec == 2 ? (cluster == 2 ? launch<P, E, 3, true, false>(g, smem, grid, st) : launch<P, E, 3, false, false>(g, smem, grid, st)) \
-                        : (cluster == 2 ? launch<P, E, 1, true, false>(g, smem, grid, st) : launch<P, E, 1, false, false>(g, smem, grid, st));
+  int grid = ctn_num_sms();
+  if (grid > g.num_items) grid = g.num_items;
+#define UM_LAUNCH(P, E)                                                                                     \
+  if (pro == P && epi == E)                                                                                 \
+    return f16 ? launch<P, E, 3, true>(g, smem, grid, st)                                                   \
+               : (nprec == 2 ? launch<P, E, 3, false>(g, smem, grid, st) : launch<P, E, 1, false>(g, smem, grid, st));
   UM_LAUNCH(PRO_NONE, EPI_RAW)
   UM_LAUNCH(PRO_DW, EPI_RAW)
   UM_LAUNCH(PRO_NONE, EPI_HEAD)

@@ -42,14 +42,6 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst_smem, const void* src, uin
                : "memory");
 }
 
-// same, multicast to every CTA of the cluster whose bit is set in cta_mask (same CTA-relative dst / mbarrier offsets)
-__device__ __forceinline__ void bulk_g2s_multicast(uint32_t dst_smem, const void* src, uint32_t bytes, uint32_t bar, uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;" ::"r"(dst_smem),
-      "l"(src), "r"(bytes), "r"(bar), "h"(cta_mask)
-      : "memory");
-}
-
 // one lane of a converged warp (elect.sync): code under this predicate is known single-threaded to the compiler, so
 // uniform-datapath instructions (tcgen05.mma / commit) are emitted without per-instruction election loops
 __device__ __forceinline__ bool elect_one() {
@@ -76,16 +68,6 @@ __device__ __forceinline__ void cluster_sync_all() {  // every thread of every C
   asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
 
-// arrive on the mbarrier at the same CTA-relative address in CTA `rank` of the cluster (release at cluster scope)
-__device__ __forceinline__ void mbar_arrive_remote(uint32_t local_bar, uint32_t rank) {
-  asm volatile(
-      "{\n\t"
-      ".reg .b32 ra;\n\t"
-      "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
-      "mbarrier.arrive.release.cluster.shared::cluster.b64 _, [ra];\n\t"
-      "}" ::"r"(local_bar), "r"(rank)
-      : "memory");
-}
 // wait with acquire at CLUSTER scope (the arrivals may come from the peer CTA)
 __device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity) {
   asm volatile(
@@ -110,17 +92,6 @@ __device__ __forceinline__ void bulk_s2peer(uint32_t dst_smem, uint32_t src_smem
       "mapa.shared::cluster.u32 rb, %3, %4;\n\t"
       "cp.async.bulk.shared::cluster.shared::cta.mbarrier::complete_tx::bytes [rd], [%1], %2, [rb];\n\t"
       "}" ::"r"(dst_smem), "r"(src_smem), "r"(bytes), "r"(bar), "r"(rank)
-      : "memory");
-}
-
-// 16-byte store into the shared memory of CTA `rank` of the cluster, same CTA-relative address (generic proxy, DSMEM)
-__device__ __forceinline__ void st_peer_v4(uint32_t local_addr, uint32_t rank, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
-  asm volatile(
-      "{\n\t"
-      ".reg .b32 ra;\n\t"
-      "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
-      "st.shared::cluster.v4.b32 [ra], {%2, %3, %4, %5};\n\t"
-      "}" ::"r"(local_addr), "r"(rank), "r"(a), "r"(b), "r"(c), "r"(d)
       : "memory");
 }
 
@@ -163,39 +134,6 @@ __device__ __forceinline__ void mma_commit(uint32_t bar) {
 // same, arriving on the barrier at this CTA-relative offset in every CTA of cta_mask
 __device__ __forceinline__ void mma_commit_multicast(uint32_t bar, uint16_t cta_mask) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-               "h"(cta_mask)
-               : "memory");
-}
-
-// ---- 2-CTA (cta_group::2) forms: one MMA spans a CTA pair (M = 256), each CTA stages its 128 rows of A and its half
-// of B; allocation / deallocation are executed by the same warp index in BOTH CTAs (verified with tools/umma_unit2.cu)
-__device__ __forceinline__ void tmem_alloc2(uint32_t smem_dst, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_dst), "r"(ncols) : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc2(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-__device__ __forceinline__ void mma2_tf32(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n\t"
-      "}" ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void mma2_f16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t"
-      "}" ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void mma2_commit_multicast(uint32_t bar, uint16_t cta_mask) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
                "h"(cta_mask)
                : "memory");
 }
@@ -251,14 +189,6 @@ __device__ __forceinline__ float to_tf32(float x) {
   return __uint_as_float(r);
 }
 
-// cheap hi/lo split for the 3xTF32 scheme (3 instructions per element instead of two emulated cvt.rna):
-//   hi = x rounded to nearest (ties away) at 10 explicit mantissa bits via integer add + mask; lo = x - hi is EXACT in
-//   fp32 and the tensor core consumes its leading tf32 bits (remaining error <= 2^-21 |x|).
-__device__ __forceinline__ void split_tf32(float x, float& hi, float& lo) {
-  hi = __uint_as_float((__float_as_uint(x) + 0x1000u) & 0xffffe000u);
-  lo = x - hi;
-}
-
 // fp16 hi/lo split of two fp32 values ("3xFP16"): hi = rn_f16(x) (saturating, never inf), lo = rn_f16(x - hi).
 // Both pieces carry 11 significant bits like TF32; packed as f16x2 (element 0 in the low half).
 __device__ __forceinline__ void split_f16x2(float x0, float x1, uint32_t& hi, uint32_t& lo) {
@@ -268,6 +198,9 @@ __device__ __forceinline__ void split_f16x2(float x0, float x1, uint32_t& hi, ui
   asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(lo) : "f"(x1 - h1), "f"(x0 - h0));
 }
 
+// cheap hi piece for the 3xTF32 scheme (3 instructions per element instead of an emulated cvt.rna): x rounded to nearest
+// (ties away) at 10 explicit mantissa bits via integer add + mask; lo = x - hi is EXACT in fp32 and the tensor core consumes
+// its leading tf32 bits (remaining error <= 2^-21 |x|).
 __device__ __forceinline__ float hi_tf32(float x) { return __uint_as_float((__float_as_uint(x) + 0x1000u) & 0xffffe000u); }
 
 // ---- descriptors -------------------------------------------------------------------------------------------------

@@ -16,7 +16,6 @@
 // 4 rows x 128 B per instruction; the loads of a group's next stage are in flight for two stage periods).
 #include "ctn_internal.h"
 #include "ctn_umma_ptx.cuh"
-#include <stdlib.h>
 #include <string.h>
 
 namespace {
@@ -35,7 +34,6 @@ struct WgArgs {
   int M, K, B, frames, pitch;
   int n_tile, tiles_n, tiles, steps_per_split, chunks, stages;
   uint32_t stage_bytes, idesc, tmem_cols;
-  int l2_prefetch;
 };
 
 struct __align__(8) WgHeader {
@@ -133,7 +131,7 @@ __global__ void __launch_bounds__(WG_THREADS, 1) k_wgrad_umma(const WgArgs g) {
     };
     static_assert(WG_KT * 4 == 128, "one step of a row is one 128-byte line");
     float4 cur[NG];
-    if (grp == 0 && g.l2_prefetch) prefetch(s0 + 2);
+    if (grp == 0) prefetch(s0 + 2);
     if (grp < nsteps) load(s0 + grp, cur);
     for (int it = grp; it < nsteps; it += 2) {
       const int s = it % g.stages;
@@ -168,7 +166,7 @@ __global__ void __launch_bounds__(WG_THREADS, 1) k_wgrad_umma(const WgArgs g) {
       ptx::fence_proxy_async_smem();
       __syncwarp();
       if (lane == 0) ptx::mbar_arrive(ptx::smem_u32(&hdr->full[s]));
-      if (grp == 0 && g.l2_prefetch && (it & 3) == 0) prefetch(s0 + it + 6);  // lines of steps it+6 .. it+9
+      if (grp == 0 && (it & 3) == 0) prefetch(s0 + it + 6);  // lines of steps it+6 .. it+9
       if (it + 2 < nsteps) load(s0 + it + 2, cur);
     }
   } else if (warp == 4) {
@@ -227,16 +225,6 @@ __global__ void __launch_bounds__(WG_THREADS, 1) k_wgrad_umma(const WgArgs g) {
   if (warp == 4) ptx::tmem_dealloc(tmem_base, g.tmem_cols);
 }
 
-int g_sms[CTN_MAX_DEVICES] = {0};  // per device ordinal
-int sms() {
-  const int dev = ctn_current_device();
-  if (g_sms[dev] == 0) {
-    cudaDeviceGetAttribute(&g_sms[dev], cudaDevAttrMultiProcessorCount, dev);
-    if (g_sms[dev] <= 0) g_sms[dev] = 148;
-  }
-  return g_sms[dev];
-}
-
 template <int NPASS>
 int launch_wg(const WgArgs& g, size_t smem, int grid, cudaStream_t st) {
   static bool attr_done[CTN_MAX_DEVICES] = {false};  // the opt-in is per device (context)
@@ -269,7 +257,7 @@ int ctn_wgrad_umma(const float* dy, size_t dy_bs, const float* x, size_t x_bs, f
   g.tiles = ((M + 127) / 128) * g.tiles_n;
   g.chunks = (frames + WG_KT - 1) / WG_KT;
   const long long total = (long long)B * g.chunks;
-  long long splits = sms() / g.tiles;
+  long long splits = ctn_num_sms() / g.tiles;
   if (splits < 1) splits = 1;
   if (splits > total) splits = total;
   g.steps_per_split = (int)((total + splits - 1) / splits);
@@ -283,8 +271,6 @@ int ctn_wgrad_umma(const float* dy, size_t dy_bs, const float* x, size_t x_bs, f
   g.idesc = ptx::make_idesc_tf32(128, g.n_tile, /*A K-major*/ 0, /*B K-major*/ 0);
   g.tmem_cols = 32;
   while ((int)g.tmem_cols < g.n_tile) g.tmem_cols <<= 1;
-  static const char* env_pf = getenv("CTN_WGRAD_PREFETCH");
-  g.l2_prefetch = env_pf ? atoi(env_pf) : 1;
   const size_t smem = WG_HEADER + 1024 + (size_t)stages * g.stage_bytes;
   const int grid = g.tiles * (int)splits;
   return nprec == 2 ? launch_wg<3>(g, smem, grid, st) : launch_wg<1>(g, smem, grid, st);

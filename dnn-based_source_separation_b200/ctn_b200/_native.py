@@ -87,9 +87,6 @@ ctn_sdr_fwd = _sig("ctn_sdr_fwd", _i, _fp, _fp, _i, _i, _f, _fp, _fp, _fp)
 ctn_sisdr_pit_bwd = _sig("ctn_sisdr_pit_bwd", _i, _fp, _fp, _fp, _i, _i, _i, _f, _fp, _fp, _f, _fp, _fp)
 ctn_last_launch_count = _sig("ctn_last_launch_count", _i)
 ctn_total_launch_count = _sig("ctn_total_launch_count", C.c_longlong)
-ctn_debug_pointwise = _sig("ctn_debug_pointwise", _i, _fp, _fp, _fp, _i, _i, _i, _i, _i, _fp, _fp, _fp, _i, _i,
-                           C.POINTER(C.c_uint32), _fp, _sz, _fp)
-ctn_debug_timeline = _sig("ctn_debug_timeline", _i, C.POINTER(C.c_ulonglong), _i)
 # DPRNN-TasNet path (cfg4) + separator stages on the pitched layout
 ctn_segment_fwd = _sig("ctn_segment_fwd", _i, _fp, _fp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _fp)
 ctn_overlap_add_fwd = _sig("ctn_overlap_add_fwd", _i, _fp, _fp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _fp)
@@ -117,7 +114,6 @@ EXPORTED = [
     "ctn_separator_fwd", "ctn_sisdr_fwd", "ctn_sisdr_pit_fwd", "ctn_sisdr_pit_scratch_bytes", "ctn_host_io_bytes",
     "ctn_convtasnet_loss_host", "ctn_train_workspace_bytes", "ctn_convtasnet_fwd_train", "ctn_convtasnet_bwd",
     "ctn_sisdr_pit_bwd", "ctn_sdr_fwd", "ctn_encoder_mc_fwd", "ctn_decoder_mc_fwd", "ctn_last_launch_count", "ctn_total_launch_count", "ctn_profile_enable", "ctn_profile_read",
-    "ctn_debug_pointwise", "ctn_debug_timeline",
     "ctn_segment_fwd", "ctn_overlap_add_fwd", "ctn_dprnn_norm_res_fwd", "ctn_stage_workspace_bytes", "ctn_sep_head_fwd", "ctn_sep_tail_fwd",
     "ctn_clip_adam_chunks", "ctn_clip_adam_step", "ctn_tcn_blocks_fwd",
     "ctn_depthwise_conv1d_fwd", "ctn_pointwise_conv1d_fwd",

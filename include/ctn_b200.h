@@ -287,18 +287,6 @@ int ctn_clip_adam_step(const int32_t* chunk_table, int n_chunks, float* const* p
                        float* exp_avg_sq, double* sumsq_scratch, const float* lr, long long* step, float beta1, float beta2, float eps,
                        float weight_decay, float max_norm, float* norm_out, ctn_stream_t stream);
 
-/* Test hook: ONE pointwise (1x1) contraction D[b][m][t] = epi(sum_k W[m][k] A[b][k][t]) in the selected numeric mode,
- * so tests can compare the tcgen05 kernels with the FFMA kernels operand by operand.  A (B,K,pitch), D (B,M,pitch),
- * pitch % 128 == 0.  epi: 0 = raw, 2 = +bias, PReLU(slope), (sum,sumsq) -> stats_out.  dbg (nullable): 4 words
- * {idesc, lbo_a, sbo_a, sbo_w} overriding the UMMA descriptors (0 = default).  workspace: >= 4*M*K*2 + 64 KiB bytes. */
-int ctn_debug_pointwise(const float* A, const float* W, float* D, int B, int M, int K, int frames, int pitch,
-                        const float* bias, const float* slope, double* stats_out, int epi, int math,
-                        const uint32_t* dbg, void* workspace, size_t workspace_bytes, ctn_stream_t stream);
-
-/* Test hook: globaltimer stamps recorded by CTA 0 of the last tcgen05 pointwise launch when the environment variable
- * CTN_UMMA_DBG has bit 128 set: [0,4096) producer, [4096,8192) MMA issuer, [8192,12288) epilogue (4 words per step). */
-int ctn_debug_timeline(unsigned long long* host, int n);
-
 /* number of kernel launches the last ctn_* call on this thread enqueued (for bench.py's gpu_launches) */
 int ctn_last_launch_count(void);
 /* kernels launched by this thread through the library since it was loaded (paths made of several entry calls: DPRNN) */

@@ -1,5 +1,5 @@
 #!/bin/bash
-# final evidence of round 2: full GPU suite, bench lines (cfg2 default, reference arm, reverse-walk A/B, cfg4), cfg4 / LSTM profiles, sanitizer
+# final evidence of round 2: full GPU suite, bench lines (cfg2 default, reference arm, cfg4), cfg4 / LSTM profiles, sanitizer
 cd "$GRAFT_REPO_ROOT" 2>/dev/null || true
 O=gpurun_out
 timeout 1800 python -m pytest -q -p no:cacheprovider tests -m gpu > $O/r02fin_pytest.log 2>&1
@@ -8,12 +8,11 @@ timeout 900 python bench.py --steps 20 --warmup 5 > $O/r02fin_bench_n1.json 2> $
 echo "bench rc=$?"; tail -2 $O/r02fin_bench_n1.err
 timeout 600 python bench.py --impl reference --steps 2 --warmup 1 > $O/r02fin_bench_ref.json 2> $O/r02fin_bench_ref.err
 echo "ref rc=$?"
-CTN_TMA_REVERSE=0 timeout 600 python bench.py --steps 20 --warmup 5 --no-cpu-baseline --no-train-block > $O/r02fin_bench_noreverse.json 2> /dev/null
 timeout 600 python bench.py --steps 20 --warmup 5 --no-cpu-baseline --no-train-block > $O/r02fin_bench_reverse.json 2> /dev/null
 timeout 600 python bench.py --config cfg4 --steps 10 --warmup 3 > $O/r02fin_cfg4.json 2> $O/r02fin_cfg4.err
 python - <<'PY'
 import json
-for n in ('bench_n1', 'bench_ref', 'bench_noreverse', 'bench_reverse', 'cfg4'):
+for n in ('bench_n1', 'bench_ref', 'bench_reverse', 'cfg4'):
     try:
         d = json.loads(open(f'gpurun_out/r02fin_{n}.json').read().strip().splitlines()[-1])
         print(n, {k: d.get(k) for k in ('value', 'ms_per_step', 'gpu_launches')}, (d.get('e2e') or {}).get('ms_per_step'), (d.get('cpu_baseline') or {}).get('value'))
